@@ -116,6 +116,51 @@ def kernel_sources_hash():
     return h.hexdigest()[:16]
 
 
+DUMP_SEED = 20241020
+DUMP_READS = 1 << 15                 # per-read results kept per batch
+DUMP_WINDOWS, DUMP_WINDOW = 16, 1024  # windows of FASTQ text kept per output stream (bytes each)
+
+
+def dump_outputs(out_dir, plan, slots, P, first_index, capacity):
+    """Writes what the last timed step computed - each slot's outputs as Plan.results / Plan.fetch_text hand them to a
+    caller - to out_dir/<name>.npy (the untimed profiling step behind the timed ones reruns the first slot's batch:
+    same outputs).  The full outputs are GBs, so beside the exact size and sha256 of every FASTQ stream only a fixed,
+    seeded sample is kept: DUMP_READS reads per batch and DUMP_WINDOWS text windows per stream.
+      read_index                  [n]            global index of each sampled read
+      read_{start,stop,dest,matched} [n, mate]   csq_read_result of those reads
+      text_bytes                  [batch, dest, mate]
+      text_sha256                 [batch, dest, mate, 8]   digest of the whole stream as big-endian 32-bit words
+      text_windows                [batch, dest, mate, window, byte]   float32 byte values, -1 past the end"""
+    import numpy as np
+
+    rng = np.random.default_rng(DUMP_SEED)
+    index, fields = [], {k: [] for k in ("start", "stop", "dest", "matched")}
+    text_bytes, sha, windows = [], [], []
+    for b, slot in enumerate(slots):
+        pick = np.sort(rng.choice(P, size=min(DUMP_READS, P), replace=False))
+        index.append(first_index + b * P + pick)
+        res = [plan.results(slot, m, P)[pick] for m in range(2)]
+        for k in fields:
+            fields[k].append(np.stack([r[k] for r in res], axis=1))
+        texts = plan.fetch_text(slot, capacity)
+        text_bytes.append([[len(t) for t in row] for row in texts])
+        sha.append([[np.frombuffer(hashlib.sha256(t).digest(), dtype=">u4") for t in row] for row in texts])
+        win = np.full((len(texts), 2, DUMP_WINDOWS, DUMP_WINDOW), -1, dtype=np.float32)
+        for d, row in enumerate(texts):
+            for m, t in enumerate(row):
+                starts = (rng.random(DUMP_WINDOWS) * max(len(t) - DUMP_WINDOW, 0)).astype(np.int64)
+                for w, s in enumerate(starts):
+                    piece = np.frombuffer(t[s : s + DUMP_WINDOW], dtype=np.uint8)
+                    win[d, m, w, : len(piece)] = piece
+        windows.append(win)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"read_index": np.concatenate(index), "text_bytes": np.array(text_bytes), "text_sha256": np.array(sha),
+              "text_windows": np.stack(windows)}
+    arrays.update({f"read_{k}": np.concatenate(v) for k, v in fields.items()})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def real_reference_available():
     """A real cutadapt 5.x + a reference tree: then the CPU arm is the reference itself (scripts/bless_against_cutadapt.py)."""
     try:
@@ -352,7 +397,9 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=60, help="timed steps; a step is one pass over the 10M-pair workload (default: ~1 s timed)")
+    ap.add_argument("--steps", type=int, default=60, help="timed steps of the headline (resident) leg; a step is one pass over the 10M-pair workload "
+                    "(default: ~1 s timed). The end-to-end legs time the same count clamped to 2..12 steps and report it "
+                    "in their own \"steps\"")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch-pairs", type=int, default=BATCH_PAIRS)
@@ -370,6 +417,8 @@ def main():
     ap.add_argument("--no-exact-stop", action="store_true", help="exact DP walks on after an error-free full match (CSQ_PLAN_NO_EXACT_STOP, A/B runs)")
     ap.add_argument("--one-stream", action="store_true", help="mate chains on one stream (CSQ_PLAN_ONE_STREAM), for A/B runs")
     ap.add_argument("--input", default="text", choices=["text", "soa"], help="batch form handed to the library")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy "
+                    "(rank 0's batches; sizes and sha256 of every output stream, a seeded sample of reads and text)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -470,6 +519,8 @@ def main():
     step_ms = ms / args.steps
     gcups_nominal = cells_per_batch * B / (step_ms * 1e-3) / 1e9
     clocks = sampler.stop(t0, t1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, plan, slots, P, rank * B * P, int(in_bytes(batches[0]) // 2 + 64 * P + 4096))
 
     # ---- end to end through the C ABI with host buffers (H2D + kernels + D2H timed); a step = B batches ----
     e2e = None

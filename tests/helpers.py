@@ -10,7 +10,6 @@ from cutseq_b200.common import BUILDIN_ADAPTERS, BarcodeConfig
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
 
 
 def manifest():
