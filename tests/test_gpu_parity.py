@@ -17,14 +17,22 @@ pytestmark = pytest.mark.gpu
 KINDS = [A.AD_BACK, A.AD_BACK_ANYWHERE, A.AD_RIGHTMOST_FRONT, A.AD_PREFIX, A.AD_SUFFIX, A.AD_NI_FRONT, A.AD_NI_BACK, A.AD_FRONT]
 
 
-def random_reads(rng, adapter, n_reads, max_len=160, alphabet="ACGT"):
+def random_reads(rng, adapter, n_reads, max_len=160, alphabet="ACGT", lengths=None, back_to_back=0.0):
+    """Reads with lengths drawn from `lengths` (default: a fixed list up to max_len) and, in 3 of 4, one or two
+    partial, mutated adapter copies at the read start, at its end or anywhere; with probability back_to_back the
+    second copy follows the first without a gap (adapter dimers)."""
+    if lengths is None:
+        lengths = [0, 1, 2, 3, 7, 20, 36, 50, 75, 100, 150, max_len]
+    else:
+        max_len = max(lengths)
     reads = []
     m = len(adapter)
     for i in range(n_reads):
-        n = rng.choice([0, 1, 2, 3, 7, 20, 36, 50, 75, 100, 150, max_len])
+        n = rng.choice(lengths)
         q = [rng.choice(alphabet + "N") if rng.random() < 0.02 else rng.choice(alphabet) for _ in range(n)]
         r = rng.random()
         if n and r < 0.75:  # plant a (partial, mutated) adapter copy, sometimes two
+            end = None  # where the previous copy ends
             for _ in range(1 + (rng.random() < 0.15)):
                 cut = rng.randint(1, m)
                 piece = list(adapter[:cut] if rng.random() < 0.5 else adapter[m - cut:])
@@ -41,7 +49,10 @@ def random_reads(rng, adapter, n_reads, max_len=160, alphabet="ACGT"):
                         piece.insert(pos, rng.choice(alphabet))
                 where = rng.random()
                 pos = 0 if where < 0.25 else (max(0, n - len(piece)) if where < 0.6 else rng.randint(0, max(0, n - 1)))
+                if end is not None and back_to_back and rng.random() < back_to_back:
+                    pos = min(end, n)
                 q[pos : pos + len(piece)] = piece
+                end = pos + len(piece)
             q = q[:max_len]
         s = "".join(q)
         if rng.random() < 0.05:

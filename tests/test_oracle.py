@@ -69,6 +69,26 @@ def test_error_thresholds():
     assert oracle.locate(p7, "TTTTTTTTTAGTTC", 0.2, BACK, 3) == (0, 5, 9, 14, 3, 1)
 
 
+def plant_copy(rng, ref, q, alpha, max_edits=3, cut=None):
+    """Overwrite part of the read q (a list) with a prefix or suffix of ref that carries up to max_edits random
+    substitutions / deletions / insertions: at the read start, at its end or anywhere."""
+    m, n = len(ref), len(q)
+    cut = rng.randint(1, m) if cut is None else cut
+    piece = list(ref[:cut] if rng.random() < 0.5 else ref[m - cut:])
+    for _ in range(rng.randint(0, max_edits)):
+        r = rng.random()
+        pos = rng.randrange(len(piece)) if piece else 0
+        if r < 0.5 and piece:
+            piece[pos] = rng.choice(alpha)
+        elif r < 0.75 and piece:
+            del piece[pos]
+        else:
+            piece.insert(pos, rng.choice(alpha))
+    pos = rng.choice([0, n - len(piece), rng.randint(0, max(0, n - len(piece)))])
+    pos = max(0, pos)
+    q[pos : pos + len(piece)] = piece
+
+
 @pytest.mark.parametrize("flags", [BACK, FRONT, PREFIX, SUFFIX, NI_FRONT, NI_BACK, ANYWHERE])
 def test_c_oracle_equals_python_restatement(flags):
     align, _ = shim_align()
@@ -80,20 +100,7 @@ def test_c_oracle_equals_python_restatement(flags):
         n = rng.choice([0, 1, 2, 5, 17, 30, 45, 60])
         q = [rng.choice(alpha + "N") for _ in range(n)]
         if n and m <= n and rng.random() < 0.7:  # plant a mutated (partial) copy
-            cut = rng.randint(1, m)
-            piece = list(ref[:cut] if rng.random() < 0.5 else ref[m - cut:])
-            for _ in range(rng.randint(0, 3)):
-                r = rng.random()
-                pos = rng.randrange(len(piece)) if piece else 0
-                if r < 0.5 and piece:
-                    piece[pos] = rng.choice(alpha)
-                elif r < 0.75 and piece:
-                    del piece[pos]
-                else:
-                    piece.insert(pos, rng.choice(alpha))
-            pos = rng.choice([0, n - len(piece), rng.randint(0, max(0, n - len(piece)))])
-            pos = max(0, pos)
-            q[pos : pos + len(piece)] = piece
+            plant_copy(rng, ref, q, alpha)
         q = "".join(q)
         rate = rng.choice([0.0, 0.1, 0.15, 0.2, 0.2, 0.34, 0.5])
         mo = rng.choice([1, 3, 3, 10, m])
@@ -101,6 +108,56 @@ def test_c_oracle_equals_python_restatement(flags):
         want = align.Aligner(ref, rate, flags=flags, min_overlap=mo).locate(q)
         got = oracle.locate(ref, q, rate, flags, mo)
         assert got == want, (ref, q, rate, flags, mo)
+
+
+def shim_adapter(kind, sequence, max_errors, min_overlap):
+    """The restated cutadapt adapter class an ALIGN op of this kind stands for."""
+    from cutseq_b200 import _abi as A
+
+    sys.path.insert(0, SHIM)
+    try:
+        from cutadapt import adapters as ad
+    finally:
+        sys.path.pop(0)
+    cls, extra = {
+        A.AD_BACK: (ad.BackAdapter, {}),
+        A.AD_BACK_ANYWHERE: (ad.BackAdapter, {"force_anywhere": True}),
+        A.AD_RIGHTMOST_FRONT: (ad.RightmostFrontAdapter, {}),
+        A.AD_PREFIX: (ad.PrefixAdapter, {}),
+        A.AD_SUFFIX: (ad.SuffixAdapter, {}),
+        A.AD_NI_FRONT: (ad.NonInternalFrontAdapter, {}),
+        A.AD_NI_BACK: (ad.NonInternalBackAdapter, {}),
+        A.AD_FRONT: (ad.FrontAdapter, {}),
+    }[kind]
+    return cls(sequence, max_errors=max_errors, min_overlap=min_overlap, **extra)
+
+
+@pytest.mark.parametrize("kind", range(1, 9))
+def test_c_oracle_equals_python_restatement_long_adapters(kind):
+    """Adapters of 64, 65, 97 and CSQ_MAX_ADAPTER bases against reads of up to CSQ_MAX_READ_LEN bases, with error
+    rates whose double rounding decides (0.29: 100 * 0.29 < 29) and absolute error counts: the whole adapter match of
+    the C oracle (count -> rate, min_overlap rules, RightmostFront's reversal) against the restated adapter classes."""
+    from cutseq_b200 import _abi as A
+    from cutseq_b200.program import Op
+
+    rng = random.Random(500 + kind)
+    for it in range(400):
+        m = rng.choice([64, 65, 97, A.CSQ_MAX_ADAPTER])
+        alpha = "ACGT" if it % 4 else "AC"
+        ref = "".join(rng.choice(alpha) for _ in range(m))
+        n = rng.choice([0, 1, m - 1, m, 150, 300, 600, A.CSQ_MAX_READ_LEN - 1, A.CSQ_MAX_READ_LEN])
+        q = [rng.choice(alpha) if rng.random() > 0.02 else "N" for _ in range(n)]
+        for _ in range(rng.choice([0, 1, 1, 2]) if n else 0):
+            plant_copy(rng, ref, q, alpha, max_edits=rng.choice([0, 3, 12, 30]), cut=m if rng.random() < 0.3 else None)
+        q = "".join(q)[:n]
+        if rng.random() < 0.05:
+            q = q.lower()
+        max_errors = rng.choice([0.0, 0.1, 0.2, 0.29, 0.35, 0.45, 1.0, 7.0, 18.0, 30.0])  # >= 1: a count
+        mo = rng.choice([1, 3, 10, m])
+        op = Op(A.OP_ALIGN, adapter_kind=kind, adapter=ref, min_overlap=mo, max_error_rate=max_errors)
+        want = shim_adapter(kind, ref, max_errors, mo).match_to(q)
+        want = None if want is None else want.as_tuple()
+        assert oracle.adapter_match(op, q) == want, (kind, ref, q, max_errors, mo)
 
 
 def test_homopolymer_equals_python_restatement():
