@@ -185,7 +185,7 @@ cudaError_t csq_launch_align(const AlignParams& p, uint32_t n_items, cudaStream_
 cudaError_t csq_launch_tail(const FinishParams& f1, const FinishParams& f2, const PairParams& p, cudaStream_t stream);  // tail.cu
 cudaError_t csq_launch_scan(uint32_t nblk, const uint32_t* block_tot, const uint32_t* block_cnt,
                             unsigned long long* block_off, unsigned long long* totals, cudaStream_t stream);
-cudaError_t csq_launch_emit(const EmitParams& p, int lanes_per_record, cudaStream_t stream);  // kernels.cu: direct, 16 lanes per record
+cudaError_t csq_launch_emit(const EmitParams& p, cudaStream_t stream);  // kernels.cu: direct, 16 lanes per record
 cudaError_t csq_launch_emit_stage(const EmitParams& p, cudaStream_t stream); // emit_stage.cu: staged through shared memory (default)
 cudaError_t csq_launch_parse(const ParseParams& p, void* tile_buf, uint16_t* masks, cudaStream_t stream);
 uint32_t csq_parse_tiles(uint64_t bytes);

@@ -1,4 +1,4 @@
-// Device helpers shared by kernels.cu and prefilter.cu: per-read interval state and the O(1) ops.
+// Device helpers shared by kernels.cu and prefilter.cu: per-read interval state, the O(1) ops and the DP column range.
 #pragma once
 
 #include "csq_internal.h"
@@ -60,6 +60,24 @@ __device__ __forceinline__ void store_state(ReadState* p, const ReadState& st) {
     q[0] = make_uint4((uint32_t)st.a | ((uint32_t)st.b << 16), st.matched, st.cp, st.cs);
     q[1] = make_uint4(st.ren_cp, st.ren_cs, (uint32_t)st.id_start | ((uint32_t)st.id_end << 16), st.qtrim);
 }
+
+// State of read idx in front of an ALIGN op: fresh for the first one, else as the previous op left it; then the
+// scalar ops between the two.
+__device__ __forceinline__ ReadState entry_state(const AlignParams& P, uint32_t idx) {
+    ReadState st = P.first ? fresh_state(P.md.seq_len[idx]) : load_state(P.md.state + idx);
+    for (int q = 0; q < P.n_pre; q++) apply_scalar(P.pre[q], st);
+    return st;
+}
+
+// DP columns min_n < j <= max_n of Aligner.locate on a read of n characters: without a free read start (siq, flags
+// bit 2) an alignment of m characters and at most k errors ends by column m + k, without a free read end (eiq, flags
+// bit 8) it starts at column n - m - k or later.
+__device__ __forceinline__ void column_range(bool siq, bool eiq, int m, int k, int n, int& min_n, int& max_n) {
+    max_n = siq ? n : min(n, m + k);
+    min_n = eiq ? 0 : max(0, n - m - k);
+}
+
+__device__ __forceinline__ csq_match no_match() { return csq_match{}; }  // found = 0, every field 0
 
 
 // 16 bytes from an arbitrary byte address: TWO aligned 128-bit loads, a select network for the word offset and four

@@ -3,7 +3,7 @@
 //   k_align<M>     exact adapter alignment, one thread per read, whole DP column in registers
 //   k_align_split  the poly-A / poly-T 100-mers: KC DP columns side by side, every column over two lanes
 //   k_scan         exclusive scan of the per-CTA totals (6 output streams, one sweep)
-//   k_emit<16>     order-preserving FASTQ text emission straight from and to global memory, 16 lanes per record:
+//   k_emit         order-preserving FASTQ text emission straight from and to global memory, 16 lanes per record:
 //                  the reverse-complementing single-end sink and the A/B partner (CSQ_PLAN_EMIT_G16) of the default
 //                  emitter k_emit_stage (emit_stage.cu)
 // (k_tail - trailing ops, quality trimming, header, name check, filters - lives in tail.cu)
@@ -34,9 +34,7 @@
 
 namespace {
 
-#ifndef CSQ_HOMO_COLUMNS
-#define CSQ_HOMO_COLUMNS 4  // DP columns a lane pair computes side by side for homopolymer adapters (k_align_split)
-#endif
+constexpr int HOMO_COLUMNS = 4;  // DP columns a lane pair computes side by side for homopolymer adapters (k_align_split)
 
 constexpr int SP_SHIFT = 10, PRIO_SHIFT = 20, COST_SHIFT = 22;
 constexpr int ORG_BIAS = 128;
@@ -118,10 +116,8 @@ __device__ __forceinline__ void last_col_update(uint32_t w, int i, int n, const 
 }
 
 __device__ __forceinline__ void best_to_match(const Best& best, int m, int n, bool reversed, csq_match& r) {
-    r.reserved = 0;
     if (best.cost == m + n + 1) {
-        r.found = 0;
-        r.ref_start = r.ref_stop = r.query_start = r.query_stop = r.score = r.errors = 0;
+        r = no_match();
         return;
     }
     int ref_start = best.origin >= 0 ? 0 : -best.origin;
@@ -135,6 +131,7 @@ __device__ __forceinline__ void best_to_match(const Best& best, int m, int n, bo
         query_stop = qe;
     }
     r.found = 1;
+    r.reserved = 0;
     r.ref_start = (int16_t)ref_start;
     r.ref_stop = (int16_t)ref_stop;
     r.query_start = (int16_t)query_start;
@@ -152,9 +149,8 @@ __device__ __forceinline__ void dp_exact(const uint8_t* __restrict__ s, int a, i
     const int k = P.k;
     const uint32_t one = P.one;
     const bool sir = P.flags & 1, siq = P.flags & 2, eir = P.flags & 4, eiq = P.flags & 8;
-    int max_n = n, min_n = 0;
-    if (!siq) max_n = min(n, M + k);
-    if (!eiq) min_n = max(0, n - M - k);
+    int min_n, max_n;
+    column_range(siq, eiq, M, k, n, min_n, max_n);
     // Column window (BACK flags, set by the prefilter): the DP starts at column j0 > min_n as if the read began
     // there.  With a free read start the cost of cell (i, j) is the best alignment of adapter[0:i] ending at j,
     // which spans at most i + cost columns; a cell that Aligner.locate can accept (cost <= k) and every
@@ -217,9 +213,8 @@ __device__ __noinline__ void dp_generic(const uint8_t* __restrict__ s, int a, in
                                         csq_match& r) {
     const int m = P.m, n = b - a, k = P.k;
     const bool sir = P.flags & 1, siq = P.flags & 2, eir = P.flags & 4, eiq = P.flags & 8;
-    int max_n = n, min_n = 0;
-    if (!siq) max_n = min(n, m + k);
-    if (!eiq) min_n = max(0, n - m - k);
+    int min_n, max_n;
+    column_range(siq, eiq, m, k, n, min_n, max_n);
     if (j0 >= 0) min_n = max(min_n, j0);  // column window, see dp_exact
     uint32_t W[CSQ_MAX_ADAPTER + 1];
     for (int i = 0; i <= m; i++) {
@@ -258,7 +253,6 @@ __device__ __noinline__ void dp_generic(const uint8_t* __restrict__ s, int a, in
     best_to_match(best, m, n, P.reversed != 0, r);
 }
 
-// M > 0: column in registers (dp_exact<M>); M == 0: any m <= CSQ_MAX_ADAPTER with the column in local memory
 // EndStatistics.adjacent_bases of cutadapt's BackAdapterStatistics.add_match: the read base in front of a 3' match
 // (match.sequence[rstart - 1 : rstart]; the read is original[a:b] here).  Slots: A, C, G, T, none, other.
 __device__ __forceinline__ void count_adjacent(const AlignParams& P, const uint8_t* s, int a, int query_start) {
@@ -270,29 +264,66 @@ __device__ __forceinline__ void count_adjacent(const AlignParams& P, const uint8
     atomicAdd(P.counters + P.adjacent_index + slot, 1ULL);
 }
 
-template <int M>
-__global__ void __launch_bounds__(128) k_align(const __grid_constant__ AlignParams P) {
-    constexpr int NW = (M > 0 ? (M + 31) / 32 : 1);
-    __shared__ uint32_t lut[M == 0 ? 1 : 256 * NW];
-    // With survivor lists: CTA c works on 128 consecutive entries of one list, the lists (longest DP first) laid
-    // end to end in units of CTAs; the grid is sized for the worst case, surplus CTAs leave at once.
-    uint32_t t = blockIdx.x * blockDim.x + threadIdx.x, count = P.n;
-    size_t list_base = 0;
+// Entry `slot` (0 .. per_cta - 1) of this CTA.  Without survivor lists CTA c takes reads c * per_cta ..; with them,
+// per_cta consecutive entries of one list, the lists (longest DP first, k_prefilter) laid end to end in units of CTAs.
+// The grid is sized for the worst case: false means the CTA has no entry at all (the same in all its threads) and
+// leaves at once.  Otherwise t < count tells whether this slot holds an entry, list_entry gives its read.
+__device__ __forceinline__ bool list_position(const AlignParams& P, uint32_t per_cta, uint32_t slot, uint32_t& t, uint32_t& count,
+                                              size_t& list_base) {
+    t = blockIdx.x * per_cta + slot;
+    count = P.n;
+    list_base = 0;
     if (P.list) {
         uint32_t cta = blockIdx.x;
         int bin = 0;
         for (; bin < CSQ_PF_BINS; bin++) {
             count = P.list_count[bin];
-            const uint32_t ctas = (count + blockDim.x - 1) / blockDim.x;
+            const uint32_t ctas = (count + per_cta - 1) / per_cta;
             if (cta < ctas) break;
             cta -= ctas;
         }
-        if (bin == CSQ_PF_BINS) return;
-        t = cta * blockDim.x + threadIdx.x;
+        if (bin == CSQ_PF_BINS) return false;
+        t = cta * per_cta + slot;
         list_base = (size_t)bin * P.n;
-    } else if (blockIdx.x * blockDim.x >= count) {
-        return;
+        return true;
     }
+    return blockIdx.x * per_cta < count;
+}
+
+// Read of entry t and the first DP column of the exact pass (j0, -1: the aligner's own min_n, see dp_exact).
+__device__ __forceinline__ uint32_t list_entry(const AlignParams& P, uint32_t t, size_t list_base, int& j0) {
+    j0 = -1;
+    if (!P.list) return t;
+    const uint32_t idx = P.list[list_base + t];
+    const uint32_t w = reinterpret_cast<const uint16_t*>(P.list + (size_t)CSQ_PF_BINS * P.n)[list_base + t];
+    if (w != 0xFFFFu) j0 = (int)w;
+    return idx;
+}
+
+// Match r of read idx (characters s): a found match sets the matched bits, counts the adjacent base and the match and
+// trims the read; then the match record and the state are stored.
+__device__ __forceinline__ void commit_match(const AlignParams& P, uint32_t idx, const uint8_t* s, const csq_match& r, ReadState st) {
+    if (r.found) {
+        st.matched |= 0x80000000u | (P.adapter_bit >= 0 ? (1u << P.adapter_bit) : 0u);
+        if (P.adjacent_index >= 0) count_adjacent(P, s, st.a, r.query_start);
+        if (P.trim_front)
+            st.a = (uint16_t)(st.a + r.query_stop);  // RemoveBeforeMatch: read[rstop:]
+        else
+            st.b = (uint16_t)(st.a + r.query_start);  // RemoveAfterMatch: read[:rstart]
+        atomicAdd(P.counters + P.counter_index, 1ULL);
+    }
+    if (P.matches) P.matches[idx] = r;
+    store_state(P.md.state + idx, st);
+}
+
+// M > 0: column in registers (dp_exact<M>); M == 0: any m <= CSQ_MAX_ADAPTER with the column in local memory
+template <int M>
+__global__ void __launch_bounds__(128) k_align(const __grid_constant__ AlignParams P) {
+    constexpr int NW = (M > 0 ? (M + 31) / 32 : 1);
+    __shared__ uint32_t lut[M == 0 ? 1 : 256 * NW];
+    uint32_t t, count;
+    size_t list_base;
+    if (!list_position(P, blockDim.x, threadIdx.x, t, count, list_base)) return;
     if constexpr (M > 0) {
         for (int c = threadIdx.x; c < 256; c += blockDim.x) {
             const int u = c & 0xDF;
@@ -303,23 +334,15 @@ __global__ void __launch_bounds__(128) k_align(const __grid_constant__ AlignPara
         __syncthreads();
     }
     if (t >= count) return;
-    uint32_t idx = t;
-    int j0 = -1;
-    if (P.list) {
-        idx = P.list[list_base + t];
-        const uint32_t w = reinterpret_cast<const uint16_t*>(P.list + (size_t)CSQ_PF_BINS * P.n)[list_base + t];
-        if (w != 0xFFFFu) j0 = (int)w;
-    }
-    ReadState st = P.first ? fresh_state(P.md.seq_len[idx]) : load_state(P.md.state + idx);
-    for (int q = 0; q < P.n_pre; q++) apply_scalar(P.pre[q], st);
+    int j0;
+    const uint32_t idx = list_entry(P, t, list_base, j0);
+    const ReadState st = entry_state(P, idx);
 
     const uint8_t* s = P.md.seq + P.md.seq_off[idx];
     csq_match r;
     if (P.count_cells) {  // nominal DP cells of this alignment, m * (max_n - min_n)  (statistics / GCUPS numerator)
-        const int n = (int)st.b - (int)st.a;
-        int max_n = n, min_n = 0;
-        if (!(P.flags & 2)) max_n = min(n, P.m + P.k);
-        if (!(P.flags & 8)) min_n = max(0, n - P.m - P.k);
+        int min_n, max_n;
+        column_range(P.flags & 2, P.flags & 8, P.m, P.k, (int)st.b - (int)st.a, min_n, max_n);
         const unsigned int mine = (unsigned int)(P.m * (max_n - min_n));
         unsigned long long* dst = P.counters + P.counter_index + (CNT_DP_CELLS - CNT_WITH_ADAPTERS);
         if (__activemask() == 0xffffffffu) {
@@ -334,17 +357,7 @@ __global__ void __launch_bounds__(128) k_align(const __grid_constant__ AlignPara
         dp_exact<M>(s, st.a, st.b, P, lut, j0, r);
     else
         dp_generic(s, st.a, st.b, P, j0, r);
-    if (r.found) {
-        st.matched |= 0x80000000u | (P.adapter_bit >= 0 ? (1u << P.adapter_bit) : 0u);
-        if (P.adjacent_index >= 0) count_adjacent(P, s, st.a, r.query_start);
-        if (P.trim_front)
-            st.a = (uint16_t)(st.a + r.query_stop);  // RemoveBeforeMatch: read[rstop:]
-        else
-            st.b = (uint16_t)(st.a + r.query_start);  // RemoveAfterMatch: read[:rstart]
-        atomicAdd(P.counters + P.counter_index, 1ULL);
-    }
-    if (P.matches) P.matches[idx] = r;
-    store_state(P.md.state + idx, st);
+    commit_match(P, idx, s, r, st);
 }
 
 // Exclusive scan over CTAs of the 8 stream totals (6 used) -> byte offset of every CTA in every
@@ -482,7 +495,6 @@ __device__ __forceinline__ void word_split(const uint8_t* dst, uint32_t len, uin
     nw = (len - head) >> 2;
 }
 
-template <int G>
 __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_emit(const __grid_constant__ EmitParams E) {
     const PairParams& P = E.pp;
     __shared__ EmitRec recs[2][CSQ_PAIR_BLOCK];
@@ -554,13 +566,14 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_emit(const __grid_constant__
     __syncthreads();
 
     // ---- phase 2 ----
-    // G lanes per record, 32 / G records side by side in a warp: the bookkeeping of a record (uniform within its
-    // group) is issued once per warp instruction for 32 / G records.  G = 16 halves the instruction count per
-    // record of the warp-per-record form (G = 32), which is bound by instruction issue.
-    constexpr int NG = 32 / G;              // records per warp pass
-    constexpr int UW = G == 32 ? 2 : G == 16 ? 3 : 5;  // unrolled word iterations: UW * G words of 4 bytes
-    constexpr int UI = 64 / G > 4 ? 4 : (G == 32 ? 2 : 2);  // unrolled id iterations: UI * G bytes
-    constexpr int MR = (23 + G - 1) / G;    // rounds over the 16 edge slots + 7 separators
+    // G = 16 lanes per record, two records side by side in a warp: the bookkeeping of a record (uniform within its
+    // group) is issued once per warp instruction for two records, half the instruction count per record of the
+    // warp-per-record form, which is bound by instruction issue.
+    constexpr int G = 16;
+    constexpr int NG = 2;   // records per warp pass
+    constexpr int UW = 3;   // unrolled word iterations: UW * G words of 4 bytes
+    constexpr int UI = 2;   // unrolled id iterations: UI * G bytes
+    constexpr int MR = 2;   // rounds over the 16 edge slots + 7 separators
     const uint32_t sl = (uint32_t)lane % G, grp = (uint32_t)lane / G;
     for (int q = 0; q < 32 / NG; q++) {
         const int slot = wid * 32 + q * NG + (int)grp;
@@ -702,49 +715,24 @@ __global__ void __launch_bounds__(128, 4) k_align_split(const __grid_constant__ 
     const uint32_t FULLM = 0xffffffffu;
     const uint32_t one = P.one;
     const int lane = threadIdx.x & 31, h = threadIdx.x & 1;
-    uint32_t t = blockIdx.x * PER_CTA + (threadIdx.x >> 1), count = P.n;
-    size_t list_base = 0;
-    if (P.list) {
-        uint32_t cta = blockIdx.x;
-        int bin = 0;
-        for (; bin < CSQ_PF_BINS; bin++) {
-            count = P.list_count[bin];
-            const uint32_t ctas = (count + PER_CTA - 1) / PER_CTA;
-            if (cta < ctas) break;
-            cta -= ctas;
-        }
-        if (bin == CSQ_PF_BINS) return;  // whole CTA
-        t = cta * PER_CTA + (threadIdx.x >> 1);
-        list_base = (size_t)bin * P.n;
-    } else if (blockIdx.x * PER_CTA >= count) {
-        return;
-    }
+    uint32_t t, count;
+    size_t list_base;
+    if (!list_position(P, PER_CTA, threadIdx.x >> 1, t, count, list_base)) return;  // whole CTA
     const bool active = t < count;  // the same for both lanes of a pair; idle pairs still take part in the shuffles
     uint32_t idx = 0;
     int j0 = -1;
     ReadState st = fresh_state(0);
     if (active) {
-        idx = t;
-        if (P.list) {
-            idx = P.list[list_base + t];
-            const uint32_t w = reinterpret_cast<const uint16_t*>(P.list + (size_t)CSQ_PF_BINS * P.n)[list_base + t];
-            if (w != 0xFFFFu) j0 = (int)w;
-        }
-        st = P.first ? fresh_state(P.md.seq_len[idx]) : load_state(P.md.state + idx);
-        for (int q = 0; q < P.n_pre; q++) apply_scalar(P.pre[q], st);
+        idx = list_entry(P, t, list_base, j0);
+        st = entry_state(P, idx);
     }
     const int a = st.a, b = st.b, n = b - a, k = P.k;
     const bool sir = P.flags & 1, siq = P.flags & 2, eir = P.flags & 4, eiq = P.flags & 8;
-    int max_n = n, min_n = 0;
-    if (!siq) max_n = min(n, M + k);
-    if (!eiq) min_n = max(0, n - M - k);
-    if (j0 >= 0) min_n = max(min_n, j0);
-    if (active && h == 0 && P.count_cells) {
-        int cmax = n, cmin = 0;
-        if (!siq) cmax = min(n, M + k);
-        if (!eiq) cmin = max(0, n - M - k);
-        atomicAdd(P.counters + P.counter_index + (CNT_DP_CELLS - CNT_WITH_ADAPTERS), (unsigned long long)(M * (cmax - cmin)));
-    }
+    int min_n, max_n;
+    column_range(siq, eiq, M, k, n, min_n, max_n);
+    if (active && h == 0 && P.count_cells)
+        atomicAdd(P.counters + P.counter_index + (CNT_DP_CELLS - CNT_WITH_ADAPTERS), (unsigned long long)(M * (max_n - min_n)));
+    if (j0 >= 0) min_n = max(min_n, j0);  // column window, see dp_exact
     const uint8_t* s = P.md.seq + (active ? P.md.seq_off[idx] : 0u);
 
     uint32_t W[MH + 1];  // local row r = global row h * MH + r
@@ -892,17 +880,7 @@ __global__ void __launch_bounds__(128, 4) k_align_split(const __grid_constant__ 
         }
         csq_match r;
         best_to_match(best, M, n, P.reversed != 0, r);
-        if (r.found) {
-            st.matched |= 0x80000000u | (P.adapter_bit >= 0 ? (1u << P.adapter_bit) : 0u);
-            if (P.adjacent_index >= 0) count_adjacent(P, P.md.seq + P.md.seq_off[idx], st.a, r.query_start);
-            if (P.trim_front)
-                st.a = (uint16_t)(st.a + r.query_stop);
-            else
-                st.b = (uint16_t)(st.a + r.query_start);
-            atomicAdd(P.counters + P.counter_index, 1ULL);
-        }
-        if (P.matches) P.matches[idx] = r;
-        store_state(P.md.state + idx, st);
+        commit_match(P, idx, P.md.seq + P.md.seq_off[idx], r, st);
     }
 }
 
@@ -945,7 +923,7 @@ cudaError_t launch_align_m(const AlignParams& p, uint32_t n_items, cudaStream_t 
             if (p.flags & 2)
                 k_align_split<M, 2><<<grid2, block, 0, stream>>>(p);
             else
-                k_align_split<M, CSQ_HOMO_COLUMNS><<<grid2, block, 0, stream>>>(p);
+                k_align_split<M, HOMO_COLUMNS><<<grid2, block, 0, stream>>>(p);
             return cudaGetLastError();
         }
     }
@@ -982,11 +960,10 @@ cudaError_t csq_launch_scan(uint32_t nblk, const uint32_t* block_tot, const uint
     return cudaGetLastError();
 }
 
-cudaError_t csq_launch_emit(const EmitParams& p, int lanes_per_record, cudaStream_t stream) {
+cudaError_t csq_launch_emit(const EmitParams& p, cudaStream_t stream) {
     if (p.pp.n == 0) return cudaSuccess;
     const dim3 grid((p.pp.n + CSQ_PAIR_BLOCK - 1) / CSQ_PAIR_BLOCK), block(CSQ_PAIR_BLOCK);
-    (void)lanes_per_record;  // 32 and 8 lanes per record were measured slower (profiles/r01_emit_variants.md) and are gone
-    k_emit<16><<<grid, block, 0, stream>>>(p);
+    k_emit<<<grid, block, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

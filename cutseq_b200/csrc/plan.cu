@@ -123,32 +123,26 @@ struct csq_plan {
 
 namespace {
 
-const char* kind_name(int k) {
-    switch (k) {
-        case CSQ_AD_BACK: return "k_align(back)";
-        case CSQ_AD_BACK_ANYWHERE: return "k_align(back,anywhere)";
-        case CSQ_AD_RIGHTMOST_FRONT: return "k_align(rightmost_front)";
-        case CSQ_AD_PREFIX: return "k_align(prefix)";
-        case CSQ_AD_SUFFIX: return "k_align(suffix)";
-        case CSQ_AD_NI_FRONT: return "k_align(noninternal_front)";
-        case CSQ_AD_NI_BACK: return "k_align(noninternal_back)";
-        case CSQ_AD_FRONT: return "k_align(front)";
-    }
-    return "k_align";
-}
+// per-kernel timer labels (csq_plan_kernel_times) of the exact aligner and the prefilter of each adapter kind
+struct KindLabels {
+    int kind;
+    const char *align, *prefilter;
+};
+constexpr KindLabels KIND_LABELS[] = {
+    {CSQ_AD_BACK, "k_align(back)", "k_prefilter(back)"},
+    {CSQ_AD_BACK_ANYWHERE, "k_align(back,anywhere)", "k_prefilter(back,anywhere)"},
+    {CSQ_AD_RIGHTMOST_FRONT, "k_align(rightmost_front)", "k_prefilter(rightmost_front)"},
+    {CSQ_AD_PREFIX, "k_align(prefix)", "k_prefilter(prefix)"},
+    {CSQ_AD_SUFFIX, "k_align(suffix)", "k_prefilter(suffix)"},
+    {CSQ_AD_NI_FRONT, "k_align(noninternal_front)", "k_prefilter(noninternal_front)"},
+    {CSQ_AD_NI_BACK, "k_align(noninternal_back)", "k_prefilter(noninternal_back)"},
+    {CSQ_AD_FRONT, "k_align(front)", "k_prefilter(front)"},
+};
 
-const char* pf_kind_name(int k) {
-    switch (k) {
-        case CSQ_AD_BACK: return "k_prefilter(back)";
-        case CSQ_AD_BACK_ANYWHERE: return "k_prefilter(back,anywhere)";
-        case CSQ_AD_RIGHTMOST_FRONT: return "k_prefilter(rightmost_front)";
-        case CSQ_AD_PREFIX: return "k_prefilter(prefix)";
-        case CSQ_AD_SUFFIX: return "k_prefilter(suffix)";
-        case CSQ_AD_NI_FRONT: return "k_prefilter(noninternal_front)";
-        case CSQ_AD_NI_BACK: return "k_prefilter(noninternal_back)";
-        case CSQ_AD_FRONT: return "k_prefilter(front)";
-    }
-    return "k_prefilter";
+KindLabels kind_labels(int kind) {
+    for (const KindLabels& l : KIND_LABELS)
+        if (l.kind == kind) return l;
+    return {kind, "k_align", "k_prefilter"};
 }
 
 // csq_op(ALIGN) -> aligner parameters (SingleAdapter.__init__ / _make_aligner of adapters.py)
@@ -245,8 +239,9 @@ int build_mate_program(const csq_op* ops, int n, int mate, MateProgram& mp) {
                 int rc = build_align(op, s.ap);
                 if (rc) return rc;
                 s.op_index = t;
-                s.name = kind_name(op.adapter_kind);
-                s.pf_name = pf_kind_name(op.adapter_kind);
+                const KindLabels labels = kind_labels(op.adapter_kind);
+                s.name = labels.align;
+                s.pf_name = labels.prefilter;
                 s.ap.n_pre = (int)pending.size();
                 for (size_t q = 0; q < pending.size(); q++) s.ap.pre[q] = pending[q];
                 pending.clear();
@@ -347,6 +342,24 @@ int ensure_common(csq_plan* plan, Slot& s, uint32_t n) {
     return 0;
 }
 
+// Per-mate arrays of a text batch of n records and `bytes` bytes of text: the record index the parse kernels build,
+// the read states and the kept match records.
+int ensure_text_index(csq_plan* plan, Slot& s, int m, uint32_t n, uint64_t bytes) {
+    int rc;
+    if ((rc = s.seq_off[m].ensure((size_t)n * 4 + 16))) return rc;
+    if ((rc = s.qual_off[m].ensure((size_t)n * 4 + 16))) return rc;
+    if ((rc = s.seq_len[m].ensure((size_t)n * 4 + 16))) return rc;
+    if ((rc = s.name_off[m].ensure((size_t)n * 4 + 16))) return rc;
+    if ((rc = s.name_end[m].ensure((size_t)n * 4 + 16))) return rc;
+    if ((rc = s.nl[m].ensure(((size_t)n * 4 + 8) * 4))) return rc;
+    if ((rc = s.masks[m].ensure(((size_t)csq_parse_tiles(bytes) + 1) * 2048))) return rc;  // 16 bits per 16-byte chunk
+    if ((rc = s.tiles[m].ensure(((size_t)csq_parse_tiles(bytes) + 4) * 8))) return rc;
+    if ((rc = s.state[m].ensure((size_t)n * sizeof(ReadState) + 32))) return rc;
+    if ((plan->flags & CSQ_PLAN_KEEP_MATCHES) && plan->prog[m].n_align)
+        if ((rc = s.matches[m].ensure((size_t)n * plan->prog[m].n_align * sizeof(csq_match) + 16))) return rc;
+    return 0;
+}
+
 // FASTQ text of a batch -> device, as it is; the record index is built by the parse kernels in enqueue_front
 int upload_text(csq_plan* plan, Slot& s, const csq_batch_text* in) {
     const uint32_t n = in->n_reads;
@@ -362,17 +375,7 @@ int upload_text(csq_plan* plan, Slot& s, const csq_batch_text* in) {
         s.text_bytes[m] = bytes;
         const size_t padded = (size_t)((bytes + 63) & ~(uint64_t)63);
         if ((rc = s.text[m].ensure(TEXT_FRONT_PAD + padded + 128))) return rc;
-        if ((rc = s.seq_off[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.qual_off[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.seq_len[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.name_off[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.name_end[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.nl[m].ensure(((size_t)n * 4 + 8) * 4))) return rc;
-        if ((rc = s.masks[m].ensure(((size_t)csq_parse_tiles(bytes) + 1) * 2048))) return rc;  // 16 bits per 16-byte chunk
-        if ((rc = s.tiles[m].ensure(((size_t)csq_parse_tiles(bytes) + 4) * 8))) return rc;
-        if ((rc = s.state[m].ensure((size_t)n * sizeof(ReadState) + 32))) return rc;
-        if ((plan->flags & CSQ_PLAN_KEEP_MATCHES) && plan->prog[m].n_align)
-            if ((rc = s.matches[m].ensure((size_t)n * plan->prog[m].n_align * sizeof(csq_match) + 16))) return rc;
+        if ((rc = ensure_text_index(plan, s, m, n, bytes))) return rc;
         uint8_t* base = (uint8_t*)s.text[m].p;
         CUDA_TRY(cudaMemsetAsync(base, 0, TEXT_FRONT_PAD, s.stream));
         // zero padding behind the text: never a line end, and readable by the 128-bit walks
@@ -437,18 +440,7 @@ int upload_bgzf(csq_plan* plan, Slot& s, const csq_batch_bgzf* in) {
     for (int m = 0; m < plan->n_mates; m++) {
         s.skip_lines[m] = in->mate[m].skip_lines;
         if ((rc = inflate_mate(plan, s, m, in->mate[m], nullptr, s.stream))) return rc;
-        const uint64_t bytes = s.text_bytes[m];
-        if ((rc = s.seq_off[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.qual_off[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.seq_len[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.name_off[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.name_end[m].ensure((size_t)n * 4 + 16))) return rc;
-        if ((rc = s.nl[m].ensure(((size_t)n * 4 + 8) * 4))) return rc;
-        if ((rc = s.masks[m].ensure(((size_t)csq_parse_tiles(bytes) + 1) * 2048))) return rc;
-        if ((rc = s.tiles[m].ensure(((size_t)csq_parse_tiles(bytes) + 4) * 8))) return rc;
-        if ((rc = s.state[m].ensure((size_t)n * sizeof(ReadState) + 32))) return rc;
-        if ((plan->flags & CSQ_PLAN_KEEP_MATCHES) && plan->prog[m].n_align)
-            if ((rc = s.matches[m].ensure((size_t)n * plan->prog[m].n_align * sizeof(csq_match) + 16))) return rc;
+        if ((rc = ensure_text_index(plan, s, m, n, s.text_bytes[m]))) return rc;
     }
     CUDA_TRY(cudaMemcpyAsync(s.totals_host + 16, s.inflate_status, sizeof(int32_t), cudaMemcpyDeviceToHost, s.stream));
     if ((rc = s.parse_misc.ensure(64))) return rc;
@@ -650,7 +642,7 @@ int enqueue_emit(csq_plan* plan, Slot& s, KernelTimer* kt, cudaStream_t st) {
         for (int m = 0; m < 2; m++) ep.out[d][m] = (uint8_t*)s.out[d][m].p;
     // default: staged through shared memory; the direct kernels stay for A/B runs and for the reverse-complementing sink
     if ((plan->flags & CSQ_PLAN_EMIT_G16) || ep.pp.revcomp)
-        CUDA_TRY(csq_launch_emit(ep, 16, st));
+        CUDA_TRY(csq_launch_emit(ep, st));
     else
         CUDA_TRY(csq_launch_emit_stage(ep, st));
     plan->launches += s.n ? 1 : 0;

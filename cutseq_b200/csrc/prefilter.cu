@@ -15,17 +15,29 @@
 // the stored state.
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "csq_internal.h"
 #include "device_common.cuh"
 
 namespace {
 
-// Survivors go to one of CSQ_PF_BINS lists (bin = class of the number of DP columns the exact pass will walk, so
-// that the 32 reads of a k_align warp have similar trip counts); list b occupies list[b * n .. b * n + count[b]).
-__device__ __forceinline__ void append_survivor(const AlignParams& P, uint32_t* __restrict__ list, uint32_t* __restrict__ list_count,
-                                                bool pass, uint32_t idx, int bin, uint32_t j0, int lane) {
+// Prologue of every prefilter kernel: the scalar ops in front of the ALIGN op run here and the state is stored, so
+// that the exact pass starts from it.
+__device__ __forceinline__ ReadState prefilter_state(const AlignParams& P, uint32_t idx) {
+    const ReadState st = entry_state(P, idx);
+    store_state(P.md.state + idx, st);
+    return st;
+}
+
+// Epilogue of every prefilter kernel, by the whole warp: the nominal DP cells of the launch (GCUPS numerator), then
+// the warp-aggregated append of the survivors.  Survivors go to one of CSQ_PF_BINS lists (bin = class of the number of
+// DP columns the exact pass will walk, so that the 32 reads of a k_align warp have similar trip counts); list b
+// occupies list[b * n .. b * n + count[b]), the first DP column j0 of each entry sits behind the lists.
+__device__ __forceinline__ void prefilter_epilogue(const AlignParams& P, uint32_t* __restrict__ list, uint32_t* __restrict__ list_count,
+                                                   unsigned int cells, bool pass, uint32_t idx, int bin, uint32_t j0) {
+    for (int o = 16; o > 0; o >>= 1) cells += __shfl_down_sync(0xffffffffu, cells, o);
+    const int lane = threadIdx.x & 31;
+    if (lane == 0 && cells) atomicAdd(P.counters + P.counter_index + (CNT_DP_CELLS - CNT_WITH_ADAPTERS), (unsigned long long)cells);
     uint16_t* __restrict__ list_j0 = reinterpret_cast<uint16_t*>(list + (size_t)CSQ_PF_BINS * P.n);
 #pragma unroll
     for (int b = 0; b < CSQ_PF_BINS; b++) {
@@ -41,6 +53,24 @@ __device__ __forceinline__ void append_survivor(const AlignParams& P, uint32_t* 
             list_j0[pos] = (uint16_t)j0;
         }
     }
+}
+
+// Column window and survivor list of a read that passed with flags 14 (BACK, RightmostFront).  fc: number of columns
+// done before the chunk in which cost[m][j] first dropped to thr[m], -1 if it never did (no row-m cell can be
+// acceptable before that chunk); smin: the smallest cost[m][j].
+__device__ __forceinline__ void window_and_bin(const AlignParams& P, int n, int min_n, int max_n, int fc, int smin, uint32_t& j0,
+                                               int& bin) {
+    // every cell Aligner.locate can accept lies in a column >= min(fc + 1, n); its value depends only on
+    // columns >= that - (m + 3k + 2)  (k_align, "column window")
+    const int jn = fc >= 0 ? fc : n;
+    const int w0 = max(min_n, jn - (P.m + 3 * P.k + 3));
+    j0 = (uint32_t)w0;
+    const int cols = max_n - w0;
+    // an error-free copy of the whole adapter (row-m cost 0 somewhere): Aligner.locate stops at that column
+    // ("exact match, stop early"), about m + 3k + 3 + 16 columns behind w0 - a list of its own, so that the
+    // warps of the exact pass that work on such reads leave together
+    const bool exact_copy = smin == 0 && P.exact_stop;
+    bin = exact_copy ? 3 : cols > 112 ? 0 : cols > 80 ? 1 : cols > 48 ? 2 : 4;  // longest first
 }
 
 // The read characters are fetched 16 columns at a time (fetch16): one thread walks 150 columns with ~10 fetches
@@ -72,16 +102,12 @@ __global__ void __launch_bounds__(256) k_prefilter(const __grid_constant__ Align
     int bin = 0;
     uint32_t j0 = 0xFFFFu;  // first DP column of the exact pass; 0xFFFF: the aligner's own min_n
     if (valid) {
-        ReadState st = P.first ? fresh_state(P.md.seq_len[idx]) : load_state(P.md.state + idx);
-        for (int q = 0; q < P.n_pre; q++) apply_scalar(P.pre[q], st);
-        store_state(P.md.state + idx, st);
-
+        const ReadState st = prefilter_state(P, idx);
         const int m = P.m, k = P.k;
         const int a = st.a, b = st.b, n = b - a;
         const bool siq = P.flags & 2, eir = P.flags & 4, eiq = P.flags & 8;
-        int max_n = n, min_n = 0;
-        if (!siq) max_n = min(n, m + k);
-        if (!eiq) min_n = max(0, n - m - k);
+        int min_n, max_n;
+        column_range(siq, eiq, m, k, n, min_n, max_n);
         cells = (unsigned int)(m * (max_n - min_n));
 
         // column min_n: cost[i] = i (vertical deltas all +1) unless the adapter start is free (all 0)
@@ -218,30 +244,10 @@ __global__ void __launch_bounds__(256) k_prefilter(const __grid_constant__ Align
                 }
             }
         }
-        if (!pass && P.matches) {
-            csq_match r;
-            r.found = r.ref_start = r.ref_stop = r.query_start = r.query_stop = r.score = r.errors = r.reserved = 0;
-            P.matches[idx] = r;
-        }
-        if (pass && window) {
-            // every cell Aligner.locate can accept lies in a column >= min(fc + 1, n); its value depends only on
-            // columns >= that - (m + 3k + 2)  (k_align, "column window")
-            const int jn = fc >= 0 ? fc : n;
-            const int w0 = max(min_n, jn - (m + 3 * k + 3));
-            j0 = (uint32_t)w0;
-            const int cols = max_n - w0;
-            // an error-free copy of the whole adapter (row-m cost 0 somewhere): Aligner.locate stops at that column
-            // ("exact match, stop early"), about m + 3k + 3 + 16 columns behind w0 - a list of its own, so that the
-            // warps of the exact pass that work on such reads leave together
-            const bool exact_copy = smin == 0 && P.exact_stop;
-            bin = exact_copy ? 3 : cols > 112 ? 0 : cols > 80 ? 1 : cols > 48 ? 2 : 4;  // longest first
-        }
+        if (!pass && P.matches) P.matches[idx] = no_match();
+        if (pass && window) window_and_bin(P, n, min_n, max_n, fc, smin, j0, bin);
     }
-    // nominal DP cells of the launch (GCUPS numerator) and warp-aggregated append of the survivors
-    for (int o = 16; o > 0; o >>= 1) cells += __shfl_down_sync(0xffffffffu, cells, o);
-    const int lane = threadIdx.x & 31;
-    if (lane == 0 && cells) atomicAdd(P.counters + P.counter_index + (CNT_DP_CELLS - CNT_WITH_ADAPTERS), (unsigned long long)cells);
-    append_survivor(P, list, list_count, pass, idx, bin, j0, lane);
+    prefilter_epilogue(P, list, list_count, cells, pass, idx, bin, j0);
 }
 
 
@@ -258,7 +264,7 @@ __global__ void __launch_bounds__(256) k_prefilter(const __grid_constant__ Align
 //   pipe, and cost[m][j] - m = up - dn is one more mad.lo; only the running minimum is an ALU instruction;
 // * adds and shifts are written as mad.lo with multipliers that come in as kernel arguments, so that ptxas cannot
 //   fold them back into ALU-pipe forms.
-// Same necessary condition, same survivor lists, same column window as k_prefilter<1, REV, false, *>.
+// Same necessary condition, same survivor lists, same column window as k_prefilter with SIR = false.
 __device__ __forceinline__ uint32_t imad_lo(uint32_t a, uint32_t b, uint32_t c) {
     uint32_t d;
     asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
@@ -270,8 +276,7 @@ __device__ __forceinline__ uint32_t imad_hi(uint32_t a, uint32_t b, uint32_t c) 
     return d;
 }
 
-// TRACK: how the row-m cost is followed - 0: mad.hi counters (FMA pipe), 1: shifts + a three-input add (ALU pipe)
-template <bool REV, int TRACK>
+template <bool REV>
 __global__ void __launch_bounds__(256) k_prefilter_fs(const __grid_constant__ AlignParams P, uint32_t* __restrict__ list,
                                                       uint32_t* __restrict__ list_count, const uint32_t one, const uint32_t two,
                                                       const uint32_t four, const uint32_t minus_one) {
@@ -292,9 +297,7 @@ __global__ void __launch_bounds__(256) k_prefilter_fs(const __grid_constant__ Al
     int bin = 0;
     uint32_t j0 = 0xFFFFu;
     if (valid) {
-        ReadState st = P.first ? fresh_state(P.md.seq_len[idx]) : load_state(P.md.state + idx);
-        for (int q = 0; q < P.n_pre; q++) apply_scalar(P.pre[q], st);
-        store_state(P.md.state + idx, st);
+        const ReadState st = prefilter_state(P, idx);
         const int k = P.k;
         const int a = st.a, b = st.b, n = b - a;
         const int max_n = n, min_n = 0;  // flags 14: read start and read end are free
@@ -322,16 +325,10 @@ __global__ void __launch_bounds__(256) k_prefilter_fs(const __grid_constant__ Al
         // (A first form only counted per chunk and re-walked "suspicious" chunks column by column: one suspicious
         // lane makes its whole warp walk again, 24 instead of 17 instructions per column on average.)
         uint32_t up = 0, dn = 0;
-        int rel = 0;  // TRACK 1: cost[m][j] - m
         auto follow = [&](uint32_t Ph, uint32_t Mh) {
-            if (TRACK == 0) {
-                up = imad_hi(Ph, two, up);
-                dn = imad_hi(Mh, two, dn);
-                smin = min(smin, (int)imad_lo(dn, minus_one, up));
-            } else {
-                rel += (int)(Ph >> 31) - (int)(Mh >> 31);
-                smin = min(smin, rel);
-            }
+            up = imad_hi(Ph, two, up);
+            dn = imad_hi(Mh, two, dn);
+            smin = min(smin, (int)imad_lo(dn, minus_one, up));
         };
         auto chunk16 = [&](const uint32_t (&w4)[4]) {
 #pragma unroll
@@ -400,24 +397,10 @@ __global__ void __launch_bounds__(256) k_prefilter_fs(const __grid_constant__ Al
                 }
             }
         }
-        if (!pass && P.matches) {
-            csq_match r;
-            r.found = r.ref_start = r.ref_stop = r.query_start = r.query_stop = r.score = r.errors = r.reserved = 0;
-            P.matches[idx] = r;
-        }
-        if (pass) {  // column window and survivor class, as in k_prefilter
-            const int jn = fc >= 0 ? fc : n;
-            const int w0 = max(min_n, jn - (m + 3 * k + 3));
-            j0 = (uint32_t)w0;
-            const int cols = max_n - w0;
-            const bool exact_copy = smin == 0 && P.exact_stop;
-            bin = exact_copy ? 3 : cols > 112 ? 0 : cols > 80 ? 1 : cols > 48 ? 2 : 4;
-        }
+        if (!pass && P.matches) P.matches[idx] = no_match();
+        if (pass) window_and_bin(P, n, min_n, max_n, fc, smin, j0, bin);
     }
-    for (int o = 16; o > 0; o >>= 1) cells += __shfl_down_sync(0xffffffffu, cells, o);
-    const int lane = threadIdx.x & 31;
-    if (lane == 0 && cells) atomicAdd(P.counters + P.counter_index + (CNT_DP_CELLS - CNT_WITH_ADAPTERS), (unsigned long long)cells);
-    append_survivor(P, list, list_count, pass, idx, bin, j0, lane);
+    prefilter_epilogue(P, list, list_count, cells, pass, idx, bin, j0);
 }
 
 template <int NW, bool REV, bool SIR>
@@ -431,16 +414,18 @@ void launch_pf(const AlignParams& p, uint32_t* list, uint32_t* list_count, dim3 
     k_prefilter<NW, REV, SIR, false><<<grid, block, 0, stream>>>(p, list, list_count);
 }
 
+// RightmostFront is the only reversed kind and has flags 14 (SIR = 0); with m <= 32 it takes k_prefilter_fs, so the
+// reversed walk is only instantiated without SIR and for NW >= 2.
 template <int NW>
 void launch_pf_nw(const AlignParams& p, uint32_t* list, uint32_t* list_count, dim3 grid, dim3 block, cudaStream_t stream) {
-    const bool sir = (p.flags & 1) != 0;
-    if (p.reversed) {
-        if (sir) launch_pf<NW, true, true>(p, list, list_count, grid, block, stream);
-        else launch_pf<NW, true, false>(p, list, list_count, grid, block, stream);
-    } else {
-        if (sir) launch_pf<NW, false, true>(p, list, list_count, grid, block, stream);
-        else launch_pf<NW, false, false>(p, list, list_count, grid, block, stream);
+    if constexpr (NW >= 2) {
+        if (p.reversed) {
+            launch_pf<NW, true, false>(p, list, list_count, grid, block, stream);
+            return;
+        }
     }
+    if (p.flags & 1) launch_pf<NW, false, true>(p, list, list_count, grid, block, stream);
+    else launch_pf<NW, false, false>(p, list, list_count, grid, block, stream);
 }
 
 // Homopolymer adapters (the poly-A / poly-T 100-mers of reference run.py:389-404, 674-707) in their two
@@ -458,9 +443,7 @@ __global__ void __launch_bounds__(256) k_prefilter_homo(const __grid_constant__ 
     unsigned int cells = 0;
     int bin = 0;
     if (valid) {
-        ReadState st = P.first ? fresh_state(P.md.seq_len[idx]) : load_state(P.md.state + idx);
-        for (int q = 0; q < P.n_pre; q++) apply_scalar(P.pre[q], st);
-        store_state(P.md.state + idx, st);
+        const ReadState st = prefilter_state(P, idx);
         const int m = P.m, k = P.k;
         const int a = st.a, b = st.b, n = b - a;
         const int span = min(n, m + k);  // columns the aligner visits (max_n - min_n for both kinds)
@@ -493,16 +476,9 @@ __global__ void __launch_bounds__(256) k_prefilter_homo(const __grid_constant__ 
             }
             bin = cols > 80 ? 0 : cols > 48 ? 1 : cols > 32 ? 2 : 4;  // longest first (list 3 is not used here)
         }
-        if (!pass && P.matches) {
-            csq_match r;
-            r.found = r.ref_start = r.ref_stop = r.query_start = r.query_stop = r.score = r.errors = r.reserved = 0;
-            P.matches[idx] = r;
-        }
+        if (!pass && P.matches) P.matches[idx] = no_match();
     }
-    for (int o = 16; o > 0; o >>= 1) cells += __shfl_down_sync(0xffffffffu, cells, o);
-    const int lane = threadIdx.x & 31;
-    if (lane == 0 && cells) atomicAdd(P.counters + P.counter_index + (CNT_DP_CELLS - CNT_WITH_ADAPTERS), (unsigned long long)cells);
-    append_survivor(P, list, list_count, pass, idx, bin, 0xFFFFu, lane);
+    prefilter_epilogue(P, list, list_count, cells, pass, idx, bin, 0xFFFFu);
 }
 
 }  // namespace
@@ -514,15 +490,9 @@ cudaError_t csq_launch_prefilter(const AlignParams& p, uint32_t* list, uint32_t*
         k_prefilter_homo<<<grid, block, 0, stream>>>(p, list, list_count);
         return cudaGetLastError();
     }
-    if (p.flags == 14 && p.m <= 32 && !getenv("CSQ_PREFILTER_V1")) {  // BACK / RightmostFront: the two-pipe form
-        static const int track = getenv("CSQ_PF_TRACK") ? atoi(getenv("CSQ_PF_TRACK")) : 0;
-        if (p.reversed) {
-            if (track) k_prefilter_fs<true, 1><<<grid, block, 0, stream>>>(p, list, list_count, 1u, 2u, 4u, 0xFFFFFFFFu);
-            else k_prefilter_fs<true, 0><<<grid, block, 0, stream>>>(p, list, list_count, 1u, 2u, 4u, 0xFFFFFFFFu);
-        } else {
-            if (track) k_prefilter_fs<false, 1><<<grid, block, 0, stream>>>(p, list, list_count, 1u, 2u, 4u, 0xFFFFFFFFu);
-            else k_prefilter_fs<false, 0><<<grid, block, 0, stream>>>(p, list, list_count, 1u, 2u, 4u, 0xFFFFFFFFu);
-        }
+    if (p.flags == 14 && p.m <= 32) {  // BACK / RightmostFront: the two-pipe form
+        if (p.reversed) k_prefilter_fs<true><<<grid, block, 0, stream>>>(p, list, list_count, 1u, 2u, 4u, 0xFFFFFFFFu);
+        else k_prefilter_fs<false><<<grid, block, 0, stream>>>(p, list, list_count, 1u, 2u, 4u, 0xFFFFFFFFu);
         return cudaGetLastError();
     }
     switch ((p.m + 31) / 32) {

@@ -1,14 +1,10 @@
 """The adapter aligner across its whole range: every adapter length class up to CSQ_MAX_ADAPTER, reads up to
 CSQ_MAX_READ_LEN, every kernel variant of the dispatch (k_align<M> with the column in registers, k_align<0> with the
 column in local memory, k_align_split for homopolymer 100-mers; k_prefilter with 1-4 bit-vector words,
-k_prefilter_fs, k_prefilter_homo and the older k_prefilter<1> form) against the CPU oracle.  Bit-exact: every
-comparison is ==."""
+k_prefilter_fs, k_prefilter_homo) against the CPU oracle.  Bit-exact: every comparison is ==."""
 
 import math
-import os
 import random
-import subprocess
-import sys
 from fractions import Fraction
 
 import pytest
@@ -21,14 +17,12 @@ from tests.test_gpu_parity import KINDS, check_locate, compare_with_oracle, rand
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MAX_M, MAX_N = A.CSQ_MAX_ADAPTER, A.CSQ_MAX_READ_LEN
 # register-resident lengths 1..34 (1, 21 / 22 and 32 are where the prefilter changes form), the local-memory DP from
 # 35 on, and the word boundaries of the bit vectors and of peq: the row-m bit (m - 1) & 31 is bit 31 or bit 0 of the
 # last word at m = 32, 33, 64, 65, 96, 97, 128
 SWEEP_M = [1, 2, 4, 7, 16, 21, 22, 31, 32, 33, 34, 35, 48, 63, 64, 65, 66, 80, 95, 96, 97, 99, 100, 101, MAX_M - 1, MAX_M]
 SWEEP_RATES = [0.0, 0.1, 0.2, 0.35]
-BACK_LIKE = (A.AD_BACK, A.AD_RIGHTMOST_FRONT)  # flags 14: the kinds of k_prefilter_fs and of the column window
 KIND_IDS = {A.AD_BACK: "back", A.AD_BACK_ANYWHERE: "back_anywhere", A.AD_RIGHTMOST_FRONT: "rightmost_front",
             A.AD_PREFIX: "prefix", A.AD_SUFFIX: "suffix", A.AD_NI_FRONT: "ni_front", A.AD_NI_BACK: "ni_back",
             A.AD_FRONT: "front"}
@@ -78,33 +72,6 @@ def test_length_sweep(m):
     for kind in KINDS:
         op, reads = sweep_case(m, kind)
         check_locate(op, reads)
-
-
-@pytest.mark.parametrize("m", [m for m in SWEEP_M if m <= 32], ids=[f"m{m}" for m in SWEEP_M if m <= 32])
-def test_prefilter_v1(m, monkeypatch):
-    """BACK / RightmostFront with m <= 32 through the older k_prefilter<1> form (CSQ_PREFILTER_V1, read per launch)
-    instead of k_prefilter_fs."""
-    monkeypatch.setenv("CSQ_PREFILTER_V1", "1")
-    for kind in BACK_LIKE:
-        op, reads = sweep_case(m, kind)
-        check_locate(op, reads)
-
-
-def test_prefilter_fs_alu_tracking():
-    """k_prefilter_fs with the row-m cost followed on the ALU pipe (CSQ_PF_TRACK=1).  The variable is read once per
-    process, so the cases run in a child process."""
-    code = (f"import sys; sys.path.insert(0, {ROOT!r})\n"
-            "from tests import test_gpu_align_matrix as t\n"
-            "for m in t.SWEEP_M:\n"
-            "    if m <= 32:\n"
-            "        for kind in t.BACK_LIKE:\n"
-            "            t.check_locate(*t.sweep_case(m, kind))\n"
-            "print('tracked ok')\n")
-    env = dict(os.environ, CSQ_PF_TRACK="1")
-    env.pop("CSQ_PREFILTER_V1", None)
-    flags = ["-s"] if sys.flags.no_user_site else []
-    p = subprocess.run([sys.executable, *flags, "-c", code], env=env, cwd=ROOT, capture_output=True, text=True, timeout=600)
-    assert p.returncode == 0 and "tracked ok" in p.stdout, p.stdout[-3000:] + p.stderr[-3000:]
 
 
 def mutate(rng, piece, subs, indel=None):
