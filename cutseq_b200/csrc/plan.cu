@@ -174,7 +174,9 @@ int build_align(const csq_op& op, AlignParams& ap) {
     ap.trim_front = front;
     ap.min_overlap = mo;
     ap.k = (int)(rate * m);
-    ap.adapter_bit = (op.adapter_id >= 0 && op.adapter_id <= 30) ? op.adapter_id : -1;
+    // bit 31 of the matched set means "any adapter matched"
+    if (op.adapter_id < -1 || op.adapter_id > 30) return fail(CSQ_ERR_INVALID, "adapter_id %d outside -1..30", op.adapter_id);
+    ap.adapter_bit = op.adapter_id;
     for (int L = 0; L <= m; L++) {
         // largest integer cost with cost <= L * rate in IEEE double, as Aligner.locate compares
         double lim = L * rate;
@@ -215,6 +217,8 @@ int build_mate_program(const csq_op* ops, int n, int mate, MateProgram& mp) {
                 if (mp.has_rename) return fail(CSQ_ERR_INVALID, "op %d: STRIP_SUFFIX must come before RENAME", t);
                 if (mp.fin.n_suffix >= 4 || op.suffix_len < 0 || op.suffix_len > CSQ_MAX_SUFFIX)
                     return fail(CSQ_ERR_INVALID, "op %d: too many / too long name suffixes", t);
+                // SuffixRemover("") would empty every name (name[:-0]); nothing implements that, so it is refused
+                if (op.suffix_len == 0) return fail(CSQ_ERR_INVALID, "op %d: empty name suffix", t);
                 mp.fin.suffix_len[mp.fin.n_suffix] = op.suffix_len;
                 memcpy(mp.fin.suffix[mp.fin.n_suffix], op.suffix, (size_t)op.suffix_len);
                 mp.fin.n_suffix++;
@@ -321,6 +325,11 @@ int validate_batch(const csq_plan* plan, const csq_batch_in* in) {
         uint32_t mx = 0;
         for (uint32_t i = 0; i < in->n_reads; i++) mx = mi.seq_len[i] > mx ? mi.seq_len[i] : mx;
         if (mx > CSQ_MAX_READ_LEN) return fail(CSQ_ERR_LIMIT, "mate %d: read of %u bases exceeds the supported %d", m + 1, mx, CSQ_MAX_READ_LEN);
+        // the id fields of the per-read state are 16 bits wide (the text path checks the same in k_tail)
+        for (uint32_t i = 0; i < in->n_reads; i++)
+            if (mi.name_off[i + 1] - mi.name_off[i] > 65535u)
+                return fail(CSQ_ERR_LIMIT, "mate %d: header of record %u (%u bytes) exceeds the supported 65535 bytes", m + 1, i,
+                            mi.name_off[i + 1] - mi.name_off[i]);
     }
     return 0;
 }

@@ -432,8 +432,10 @@ void launch_pf_nw(const AlignParams& p, uint32_t* list, uint32_t* list_count, di
 // non-internal kinds need no bit-vectors.  With e(l) = number of read characters different from the adapter
 // base among the l characters next to the anchored end (read start for NonInternalFront, read end for
 // NonInternalBack), every alignment that covers those l characters costs at least e(l), and covers at most
-// l + cost adapter characters; thr[] grows by at most 1 per step, so "cost <= thr[min(m, l + cost)]" can
-// only hold for some cost >= e(l) if it holds for cost == e(l).  e(l) never decreases, hence the scan
+// l + cost adapter characters.  An alignment of length >= min_overlap needs cost >= min_overlap - l as well (a
+// read shorter than min_overlap can still be covered by min_overlap adapter characters, with deletions), so the
+// cost is at least c = max(e(l), min_overlap - l); thr[] grows by at most 1 per step, so "cost <= thr[min(m, l +
+// cost)]" can only hold for some cost >= c if it holds for cost == c.  e(l) never decreases, hence the scan
 // stops at the first l with e(l) > k (about 20 characters into a random read instead of m + k = 115 columns).
 __global__ void __launch_bounds__(256) k_prefilter_homo(const __grid_constant__ AlignParams P, uint32_t* __restrict__ list,
                                                         uint32_t* __restrict__ list_count) {
@@ -456,8 +458,8 @@ __global__ void __launch_bounds__(256) k_prefilter_homo(const __grid_constant__ 
         for (; l <= span; l++) {
             e += ((cw.next() & 0xDFu) != (uint32_t)P.letter) ? 1 : 0;
             if (e > k) break;
-            const int L = min(m, l + e);
-            if (L >= P.min_overlap && e <= (int)P.thr[L]) {
+            const int c = max(e, P.min_overlap - l);
+            if (c <= (int)P.thr[min(m, l + c)]) {
                 pass = true;
                 break;
             }

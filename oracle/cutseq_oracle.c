@@ -264,12 +264,16 @@ static int adjacent_slot(const char* seq, int query_start) {
 }
 
 /* ---- per-read working record (the SequenceRecord + ModificationInfo of one mate) ---- */
+/* Longest name a record can carry: the product's 65535-byte header limit, then a renamed id of at most that length
+ * plus '_' and two UMI parts of at most CSQ_MAX_READ_LEN bases each. */
+#define ORC_NAME_CAP (65535 + 1 + 2 * CSQ_MAX_READ_LEN)
+
 typedef struct orc_read {
     char* seq;   /* working copies, sliced by moving seq/qual and len */
     char* qual;
     int len;
     int orig_off; /* offset of seq[0] inside the original read (undefined after REVCOMP) */
-    char name[4096];
+    char* name; /* ORC_NAME_CAP bytes, owned by the chunk worker */
     int name_len;
     /* ModificationInfo */
     int n_matches;
@@ -394,11 +398,10 @@ static void apply_single(const csq_op* op, orc_read* r, orc_match* match_out, ui
     }
 }
 
-/* Renamer / PairedEndRenamer with the templates run.py builds. */
-static int apply_rename(const csq_op* op, orc_read* r, const orc_read* r1, const orc_read* r2) {
+/* Renamer / PairedEndRenamer with the templates run.py builds; out: ORC_NAME_CAP bytes of scratch. */
+static int apply_rename(const csq_op* op, orc_read* r, const orc_read* r1, const orc_read* r2, char* out) {
     int s, e;
     parse_name_id(r->name, r->name_len, &s, &e);
-    char out[4096];
     int n = 0;
     memcpy(out, r->name + s, (size_t)(e - s));
     n = e - s;
@@ -451,7 +454,7 @@ static void write_fastq(orc_buf* b, const orc_read* r) { /* dnaio: @name\nseq\n+
     b->records++;
 }
 
-static void load_read(orc_read* r, const csq_mate_in* in, uint32_t i) {
+static void load_read(orc_read* r, const csq_mate_in* in, uint32_t i, char* name_buf) {
     int len = (int)in->seq_len[i];
     r->buf_seq = (char*)malloc((size_t)len + 1);
     r->buf_qual = (char*)malloc((size_t)len + 1);
@@ -464,8 +467,9 @@ static void load_read(orc_read* r, const csq_mate_in* in, uint32_t i) {
     r->qual = r->buf_qual;
     r->len = len;
     r->orig_off = 0;
+    r->name = name_buf;
     r->name_len = (int)(in->name_off[i + 1] - in->name_off[i]);
-    if (r->name_len > 4000) r->name_len = 4000;
+    if (r->name_len > 65535) r->name_len = 65535; /* orc_run_batch reports CSQ_ERR_LIMIT, as the product does */
     memcpy(r->name, in->name + in->name_off[i], (size_t)r->name_len);
     r->n_matches = 0;
     r->matched_ids = 0;
@@ -479,7 +483,8 @@ static void load_read(orc_read* r, const csq_mate_in* in, uint32_t i) {
  * steps: TooShort filter ("any" mate), optional IsUntrimmedAny filter ("any"), sink.
  * Outputs: FASTQ text per destination and mate (malloc'ed into out->text[][].data, caller
  * frees with orc_free), optional per-mate results and per-op matches.
- * Returns 0, or CSQ_ERR_PAIRING when mate ids differ at a paired RENAME.
+ * Returns 0, CSQ_ERR_PAIRING when mate ids differ at a paired RENAME, or CSQ_ERR_LIMIT for a header longer than
+ * 65535 bytes.
  */
 typedef struct orc_job {
     const csq_op *ops1, *ops2;
@@ -514,12 +519,15 @@ static void* chunk_worker(void* arg) {
         if (ops1[t].kind == CSQ_OP_ALIGN) first_align[0] = t;
         if (paired && ops2[t].kind == CSQ_OP_ALIGN) first_align[1] = t;
     }
+    char* names = (char*)malloc((size_t)3 * ORC_NAME_CAP); /* mate 1, mate 2, rename scratch */
     for (uint32_t i = J->lo; i < J->hi; i++) {
         orc_read r[2];
-        load_read(&r[0], &in->mate[0], i);
-        if (paired) load_read(&r[1], &in->mate[1], i);
+        load_read(&r[0], &in->mate[0], i, names);
+        if (paired) load_read(&r[1], &in->mate[1], i, names + ORC_NAME_CAP);
         /* dnaio's paired reader: "Records are improperly paired" unless r1.is_mate(r2) */
         if (paired && !names_match(r[0].name, r[0].name_len, r[1].name, r[1].name_len)) J->status = CSQ_ERR_PAIRING;
+        for (int mt_i = 0; mt_i < (paired ? 2 : 1); mt_i++)
+            if (in->mate[mt_i].name_off[i + 1] - in->mate[mt_i].name_off[i] > 65535u) J->status = CSQ_ERR_LIMIT;
         k->n++;
         k->total_bp[0] += (uint64_t)r[0].len;
         if (paired) k->total_bp[1] += (uint64_t)r[1].len;
@@ -530,10 +538,10 @@ static void* chunk_worker(void* arg) {
                      * record_names_match(read1.name, read2.name); each mate then keeps its OWN id */
                     if (!names_match(r[0].name, r[0].name_len, r[1].name, r[1].name_len)) J->status = CSQ_ERR_PAIRING;
                     orc_read a = r[0], bb = r[1]; /* both names are built from the pre-rename infos */
-                    apply_rename(&ops1[t], &r[0], &a, &bb);
-                    apply_rename(&ops2[t], &r[1], &a, &bb);
+                    apply_rename(&ops1[t], &r[0], &a, &bb, names + 2 * ORC_NAME_CAP);
+                    apply_rename(&ops2[t], &r[1], &a, &bb, names + 2 * ORC_NAME_CAP);
                 } else {
-                    apply_rename(&ops1[t], &r[0], NULL, NULL);
+                    apply_rename(&ops1[t], &r[0], NULL, NULL, names + 2 * ORC_NAME_CAP);
                 }
                 continue;
             }
@@ -589,6 +597,7 @@ static void* chunk_worker(void* arg) {
             free(r[mt_i].buf_qual);
         }
     }
+    free(names);
     return NULL;
 }
 

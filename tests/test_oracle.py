@@ -263,3 +263,134 @@ def test_pinning_status_is_honest():
         assert pin["pinned"] is False or pin["checked_against"], "PINNING.json claims a check that cannot have run here"
     else:
         assert rc == 0, "the real cutadapt disagrees with tests/golden (run scripts/bless_against_cutadapt.py)"
+
+
+def test_long_headers_come_back_whole():
+    """Headers up to the product's 65 535 bytes, with and without RENAME; a longer one is CSQ_ERR_LIMIT."""
+    from cutseq_b200 import _abi as A
+    from cutseq_b200.program import Filters, Op, Program
+
+    rng = random.Random(8)
+    for n in (4001, 20000, 65535):
+        heads = ["".join(rng.choice("abc:/") for _ in range(n)), "i" * 10 + " " + "c" * (n - 11)]
+        recs = [(h, "ACGTACGT", "IIIIIIII") for h in heads]
+        batch, keep = oracle.make_batch(recs)
+        for ops, names in (([], heads), ([Op(A.OP_RENAME)], [heads[0], "i" * 10])):
+            out = oracle.run_batch(Program(False, ops, [], Filters(0)), batch)
+            assert out["status"] == 0
+            assert [r[0] for r in oracle.parse_fastq_text(out["text"][0][0])] == names
+    batch, keep = oracle.make_batch([("x" * 65536, "ACGT", "IIII")])
+    assert oracle.run_batch(Program(False, [], [], Filters(0)), batch)["status"] == A.ERR_LIMIT
+
+
+def test_longest_renamed_name():
+    """A 65 535-byte id behind which PairedEndRenamer puts two UMI parts of 895 bases: the longest name a record
+    can get, byte for byte."""
+    from cutseq_b200 import _abi as A
+    from cutseq_b200.program import Filters, Op, Program
+
+    rng = random.Random(9)
+    n = A.CSQ_MAX_READ_LEN
+    s1, s2 = ("".join(rng.choice("ACGT") for _ in range(n)) for _ in range(2))
+    h = "".join(rng.choice("abcdefgh0123456789") for _ in range(65535))
+    ops = [Op(A.OP_CUT, length=n), Op(A.OP_RENAME, rename_parts=A.REN_R1_PREFIX | A.REN_R2_PREFIX)]
+    batch, keep = oracle.make_batch([(h, s1, "I" * n)], [(h, s2, "I" * n)])
+    out = oracle.run_batch(Program(True, ops, ops, Filters(0)), batch)
+    assert out["status"] == 0
+    for m in range(2):
+        assert out["text"][0][m] == f"@{h}_{s1}{s2}\n\n+\n\n".encode()
+
+
+def shim_modifiers():
+    sys.path.insert(0, SHIM)
+    try:
+        from cutadapt import modifiers
+        from cutadapt._record import SequenceRecord
+        from cutadapt.info import ModificationInfo
+    finally:
+        sys.path.pop(0)
+    return modifiers, SequenceRecord, ModificationInfo
+
+
+def shim_run(prog, mates):
+    """The generated program as cutadapt modifiers, per read (pair): final names, bases, qualities, destinations."""
+    from cutseq_b200 import _abi as A
+    from cutseq_b200.program import rename_template
+
+    mods, Record, Info = shim_modifiers()
+    n_mates = len(mates)
+    opss = [prog.ops_r1, prog.ops_r2][:n_mates]
+    steps = []
+    for t in range(len(opss[0])):
+        row = []
+        for ops in opss:
+            op = ops[t]
+            if op.kind == A.OP_STRIP_SUFFIX:
+                row.append(mods.SuffixRemover(op.suffix))
+            elif op.kind == A.OP_ALIGN:
+                row.append((mods.AdapterCutter([shim_adapter(op.adapter_kind, op.adapter, op.max_error_rate, op.min_overlap)]), op.adapter_id))
+            elif op.kind == A.OP_CUT:
+                row.append(mods.UnconditionalCutter(op.length))
+            elif op.kind == A.OP_QTRIM:
+                row.append(mods.QualityTrimmer(op.cutoff_front, op.cutoff_back, op.quality_base))
+            elif op.kind == A.OP_RENAME:
+                tpl = rename_template(op.rename_parts)
+                row.append(mods.PairedEndRenamer(tpl) if n_mates == 2 else mods.Renamer(tpl))
+            else:
+                raise AssertionError(op)
+        steps.append(row)
+    out = []
+    flt = prog.filters
+    for i in range(len(mates[0])):
+        reads = [Record(*mates[m][i]) for m in range(n_mates)]
+        infos = [Info(r) for r in reads]
+        matched = [0] * n_mates
+        for row in steps:
+            if isinstance(row[0], mods.PairedEndRenamer):
+                reads = list(row[0](reads[0], reads[1], infos[0], infos[1]))
+                continue
+            for m in range(n_mates):
+                mod = row[m]
+                if isinstance(mod, tuple):
+                    mod, aid = mod
+                    before = len(infos[m].matches)
+                    reads[m] = mod(reads[m], infos[m])
+                    if len(infos[m].matches) > before and aid >= 0:
+                        matched[m] |= 1 << aid
+                else:
+                    reads[m] = mod(reads[m], infos[m])
+        if any(len(r) < flt.min_length for r in reads):
+            dest = A.DEST_SHORT
+        elif flt.untrimmed_enabled and any(req & ~matched[m] for m, req in enumerate([flt.required_r1, flt.required_r2][:n_mates])):
+            dest = A.DEST_UNTRIMMED
+        else:
+            dest = A.DEST_TRIMMED
+        out.append((dest, [(r.name, r.sequence, r.qualities) for r in reads]))
+    return out
+
+
+def test_generated_programs_equal_cutadapt_modifiers():
+    """Programs of tests/program_gen.py without COND_CUT and REVCOMP (cutseq's own classes, checked by known answers
+    elsewhere) through the restated cutadapt modifiers, read by read, against oracle.run_batch."""
+    from cutseq_b200 import _abi as A
+    from tests import program_gen as G
+
+    n_reads = 0
+    for seed in range(20):
+        rng = random.Random(3300 + seed)
+        prog = G.random_program(rng, paired=seed % 2 == 1, cond_cut=False, revcomp=False)
+        mates = G.random_mates(rng, prog, 100, lengths=G.EDGE_LENGTHS[:-1] + [40, 64, 100, 150, 300])
+        batch, keep = oracle.make_batch(*mates)
+        want = oracle.run_batch(prog, batch)
+        assert want["status"] == 0
+        got = shim_run(prog, mates)
+        texts = {}
+        for d in range(A.CSQ_N_DEST):
+            for m in range(len(mates)):
+                texts[d, m] = iter(oracle.parse_fastq_text(want["text"][d][m]))
+        for i, (dest, recs) in enumerate(got):
+            assert int(want["results"][0]["dest"][i]) == dest, (seed, i)
+            for m, rec in enumerate(recs):
+                assert next(texts[dest, m]) == rec, (seed, i, m)
+        n_reads += len(got)
+    assert n_reads == 2000
