@@ -4,7 +4,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 CSQ_MAX_ADAPTER = 128
 CSQ_MAX_READ_LEN = 895
@@ -44,6 +44,7 @@ PLAN_ONE_STREAM = 64
 PLAN_EMIT_G16 = 256
 PLAN_NO_EXACT_STOP = 1024
 PLAN_GZIP_OUT = 4096
+PLAN_FASTA = 8192
 
 
 class csq_op(C.Structure):

@@ -67,6 +67,16 @@ struct ParseParams {  // FASTQ text of one mate -> record index (parse.cu)
     uint32_t* first_off;       // [1] byte offset of the first record (0 when skip == 0)
 };
 
+struct FastaParams {  // FASTA text of one mate -> record index (parse.cu, CSQ_PLAN_FASTA)
+    ParseParams p;           // p.nl: [n] offsets of the record starts; p.nl_total: record starts found
+    uint8_t* pool;           // wrapped sequences, joined: text + pool0 (one buffer, so that seq_off reaches both)
+    uint32_t pool0;
+    uint32_t* pad_len;       // [n], 16-byte aligned: padded lengths of the wrapped records, scanned into pool offsets
+    uint32_t* pool_total;    // [1]
+    uint32_t qual0;          // qual_off of every record: into the constant buffer of 'I' bytes
+};
+#define CSQ_FASTA_QUAL_BYTES 1024  /* the 'I' buffer: qual_off = 64, then CSQ_MAX_READ_LEN bytes and padding */
+
 struct AlignParams {
     MateDev md;
     csq_match* matches;    // nullable: per-read record of this ALIGN op
@@ -182,13 +192,16 @@ enum {
 
 // launchers implemented in kernels.cu (all asynchronous on `stream`)
 cudaError_t csq_launch_align(const AlignParams& p, uint32_t n_items, cudaStream_t stream);
-cudaError_t csq_launch_tail(const FinishParams& f1, const FinishParams& f2, const PairParams& p, cudaStream_t stream);  // tail.cu
+cudaError_t csq_launch_tail(const FinishParams& f1, const FinishParams& f2, const PairParams& p, bool fasta, cudaStream_t stream);  // tail.cu
 cudaError_t csq_launch_scan(uint32_t nblk, const uint32_t* block_tot, const uint32_t* block_cnt,
                             unsigned long long* block_off, unsigned long long* totals, cudaStream_t stream);
-cudaError_t csq_launch_emit(const EmitParams& p, cudaStream_t stream);  // kernels.cu: direct, 16 lanes per record
-cudaError_t csq_launch_emit_stage(const EmitParams& p, cudaStream_t stream); // emit_stage.cu: staged through shared memory (default)
+// fasta: ">name\nseq\n" records (CSQ_PLAN_FASTA)
+cudaError_t csq_launch_emit(const EmitParams& p, bool fasta, cudaStream_t stream);  // kernels.cu: direct, 16 lanes per record
+cudaError_t csq_launch_emit_stage(const EmitParams& p, bool fasta, cudaStream_t stream); // emit_stage.cu: staged through shared memory (default)
 cudaError_t csq_launch_parse(const ParseParams& p, void* tile_buf, uint16_t* masks, cudaStream_t stream);
 uint32_t csq_parse_tiles(uint64_t bytes);
+cudaError_t csq_launch_parse_fasta(const FastaParams& f, void* tile_buf, uint16_t* masks, cudaStream_t stream);
+uint32_t csq_parse_fasta_launches(uint64_t bytes, uint32_t n);
 cudaError_t csq_launch_prefilter(const AlignParams& p, uint32_t* list, uint32_t* list_count, cudaStream_t stream);
 bool csq_align_has_exact_kernel(int m);
 cudaError_t csq_launch_int_peak(int variant, int iters, unsigned int* sink, int blocks, int threads, cudaStream_t stream);

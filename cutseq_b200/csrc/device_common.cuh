@@ -143,6 +143,8 @@ struct RecordShape {
     uint32_t lenA, lenB;
 };
 
+// FASTA: ">name\nseq\n" instead of "@name\nseq\n+\nqual\n"
+template <bool FASTA = false>
 __device__ __forceinline__ RecordShape record_shape(const PairParams& P, const ReadState& own, const ReadState& r1,
                                                     const ReadState& r2) {
     RecordShape rs;
@@ -154,7 +156,7 @@ __device__ __forceinline__ RecordShape record_shape(const PairParams& P, const R
     if (P.rename_parts & CSQ_REN_R2_PREFIX) rs.lenB = r2.ren_cp & 0xFFFFu;
     rs.umi_len = (P.rename_parts ? 1u : 0u) + rs.lenA + rs.lenB;
     rs.seq_len = (uint32_t)own.b - (uint32_t)own.a;
-    rs.total = 1 + rs.id_len + rs.umi_len + 1 + rs.seq_len + 3 + rs.seq_len + 1;
+    rs.total = FASTA ? 1 + rs.id_len + rs.umi_len + 1 + rs.seq_len + 1 : 1 + rs.id_len + rs.umi_len + 1 + rs.seq_len + 3 + rs.seq_len + 1;
     return rs;
 }
 

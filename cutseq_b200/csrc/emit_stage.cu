@@ -26,7 +26,9 @@
 // Every source byte is read once and every output byte written once.  A pass that does not fit the staging
 // buffers is halved; a pair that does not fit alone (reads near the length limit with very long headers) takes
 // a bytewise path.  (The mate-name check of PairedEndRenamer / dnaio's paired reader is k_tail's, tail.cu.)  The
-// reverse-complementing single-end sink stays with k_emit<16>.
+// reverse-complementing single-end sink stays with k_emit.
+// FASTA (CSQ_PLAN_FASTA): k_emit_stage<.., .., true> writes ">name\nseq\n"; header and bases are two source spans of the
+// one text buffer (a wrapped sequence sits in the pool behind the text), there are no qualities and role-1 lanes idle.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -154,8 +156,8 @@ __device__ __forceinline__ void copy_s2s(uint8_t* sm, uint32_t s, uint32_t d, ui
 // measured and dropped: the rotation differs from lane to lane, so its four loop variants run one after the other
 // inside a warp; 0.745 ms against 0.645 ms per step, profiles/r01_emit_variants.md.)
 
-// PAIRED: two mates per pair; ONE_POOL: text batch (header, bases and qualities of a mate in one buffer)
-template <bool PAIRED, bool ONE_POOL>
+// PAIRED: two mates per pair; ONE_POOL: text batch (header, bases and qualities of a mate in one buffer); FASTA: FASTA out
+template <bool PAIRED, bool ONE_POOL, bool FASTA>
 __global__ void __launch_bounds__(CSQ_PAIR_BLOCK, 2) k_emit_stage(const __grid_constant__ EmitParams E) {
     extern __shared__ __align__(16) uint8_t es_smem[];
     __shared__ unsigned int wtot[8][ES_WARPS];  // per-stream totals of every warp
@@ -184,7 +186,7 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK, 2) k_emit_stage(const __grid_c
         st[0] = load_state(P.md[0].state + idx);
         st[1] = paired ? load_state(P.md[1].state + idx) : st[0];
         for (int mt = 0; mt < n_mates; mt++) {
-            shape[mt] = record_shape(P, st[mt], st[0], st[1]);
+            shape[mt] = record_shape<FASTA>(P, st[mt], st[0], st[1]);
             len[mt] = shape[mt].total;
         }
     }
@@ -241,7 +243,7 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK, 2) k_emit_stage(const __grid_c
     const uint8_t* const poolB = (P.rename_parts & CSQ_REN_R2_PREFIX) ? P.md[1].seq : nullptr;
     // a text batch keeps header, bases and qualities of a mate in ONE buffer: one source span per mate and pass
     constexpr bool one_pool = ONE_POOL;
-    constexpr int n_pools = ONE_POOL ? 1 : 3;
+    constexpr int n_pools = FASTA ? 2 : ONE_POOL ? 1 : 3;
 
     const int q = lane >> 1, role = lane & 1;
     constexpr int ppass = PAIRED ? 8 : 16;
@@ -396,12 +398,13 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK, 2) k_emit_stage(const __grid_c
             const uint32_t e_name = 1u + fid, e_umi = e_name + fumi, e_seq = e_umi + 1u + fl, e_qual = e_seq + 3u + fl;
             for (uint32_t p = lane; p < F.len; p += 32) {
                 uint8_t c;
-                if (p < e_name) c = p == 0 ? (uint8_t)'@' : nm[p - 1];
+                if (p < e_name) c = p == 0 ? (uint8_t)(FASTA ? '>' : '@') : nm[p - 1];
                 else if (p < e_umi) {
                     const uint32_t x = p - e_name;
                     c = x == 0 ? (uint8_t)'_' : (x - 1 < fla ? pa[x - 1] : pb[x - 1 - fla]);
                 } else if (p == e_umi) c = '\n';
                 else if (p < e_seq) c = sq[p - e_umi - 1];
+                else if (FASTA) c = '\n';
                 else if (p < e_seq + 3) c = (p - e_seq == 1) ? (uint8_t)'+' : (uint8_t)'\n';
                 else if (p < e_qual) c = ql[p - e_seq - 3];
                 else c = '\n';
@@ -454,13 +457,13 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK, 2) k_emit_stage(const __grid_c
 
         // ---- reformat ----
         const uint32_t s_id = ES_SRC0 + sd_name + R.nm;
-        if (valid) {
+        if (valid && (!FASTA || role == 0)) {
             const uint32_t d_seq = d0 + 1u + id_len + umi_len + 1u;
             const uint32_t d_qual = d_seq + seq_len + 3u;
             const uint32_t s_big = ES_SRC0 + (role ? sd_qual + R.ql : sd_seq + R.sq) + a;
             copy_s2s(sm, s_big, role ? d_qual : d_seq, seq_len);
             if (role == 0) {
-                sm[d0] = '@';
+                sm[d0] = FASTA ? '>' : '@';
                 copy_s2s(sm, s_id, d0 + 1u, id_len);
                 if (umi_len) {
                     sm[d0 + 1u + id_len] = '_';
@@ -515,21 +518,22 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK, 2) k_emit_stage(const __grid_c
     if (draining && lane == 0) bulk_wait_read();  // shared memory must outlive the reads of the last bulk stores
 }
 
-template <bool PAIRED, bool ONE_POOL>
+template <bool PAIRED, bool ONE_POOL, bool FASTA = false>
 cudaError_t launch_stage(const EmitParams& p, cudaStream_t stream) {
     // per device: a function attribute belongs to the current context
-    cudaError_t attr = cudaFuncSetAttribute(k_emit_stage<PAIRED, ONE_POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ES_WARPS * ES_WARP_BYTES));
+    cudaError_t attr = cudaFuncSetAttribute(k_emit_stage<PAIRED, ONE_POOL, FASTA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ES_WARPS * ES_WARP_BYTES));
     if (attr != cudaSuccess) return attr;
-    k_emit_stage<PAIRED, ONE_POOL><<<(p.pp.n + CSQ_PAIR_BLOCK - 1) / CSQ_PAIR_BLOCK, CSQ_PAIR_BLOCK, ES_WARPS * ES_WARP_BYTES, stream>>>(p);
+    k_emit_stage<PAIRED, ONE_POOL, FASTA><<<(p.pp.n + CSQ_PAIR_BLOCK - 1) / CSQ_PAIR_BLOCK, CSQ_PAIR_BLOCK, ES_WARPS * ES_WARP_BYTES, stream>>>(p);
     return cudaGetLastError();
 }
 
 }  // namespace
 
-cudaError_t csq_launch_emit_stage(const EmitParams& p, cudaStream_t stream) {
+cudaError_t csq_launch_emit_stage(const EmitParams& p, bool fasta, cudaStream_t stream) {
     if (p.pp.n == 0) return cudaSuccess;
     const PairParams& P = p.pp;
     const bool paired = P.n_mates == 2;
+    if (fasta) return paired ? launch_stage<true, false, true>(p, stream) : launch_stage<false, false, true>(p, stream);
     const bool one_pool = P.md[0].seq == P.md[0].name && P.md[0].seq == P.md[0].qual;
     if (paired) return one_pool ? launch_stage<true, true>(p, stream) : launch_stage<true, false>(p, stream);
     return one_pool ? launch_stage<false, true>(p, stream) : launch_stage<false, false>(p, stream);

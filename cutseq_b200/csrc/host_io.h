@@ -60,6 +60,24 @@ struct MateParser {
 // ---- text batches (text_reader.cpp) ----
 uint64_t count_newlines(const uint8_t* p, size_t n);
 uint64_t after_kth_newline(const uint8_t* p, size_t n, uint64_t k);  // offset one past the k-th '\n', UINT64_MAX if fewer
+// FASTA record starts ('>' as the first byte of a line); `prev` is the byte in front of p ('\n' at a line start)
+uint64_t count_fasta_records(const uint8_t* p, size_t n, uint8_t prev);
+uint64_t kth_fasta_record(const uint8_t* p, size_t n, uint64_t k, uint8_t prev);  // offset of the k-th (k >= 1), UINT64_MAX if fewer
+
+// How a byte stream is cut into batches of whole records: FASTQ after 4 k line ends, FASTA in front of the (k + 1)-th
+// record start.  Counts and cuts work on pieces of the stream; `prev` is the byte in front of a piece.
+struct RecordCut {
+    bool fasta = false;
+    uint64_t target(uint32_t max_reads) const { return fasta ? (uint64_t)max_reads + 1 : 4ull * max_reads; }
+    uint64_t count(const uint8_t* p, size_t n, uint8_t prev) const {
+        return fasta ? count_fasta_records(p, n, prev) : count_newlines(p, n);
+    }
+    uint64_t cut(const uint8_t* p, size_t n, uint64_t k, uint8_t prev) const {
+        return fasta ? kth_fasta_record(p, n, k, prev) : after_kth_newline(p, n, k);
+    }
+    // a piece counted without its `prev` (pieces counted side by side): the record start it may hold at offset 0
+    uint64_t edge(const uint8_t* p, size_t n, uint8_t prev) const { return fasta && n && p[0] == '>' && prev == '\n' ? 1 : 0; }
+};
 
 // gzip / DEFLATE decoder (inflate.cpp): whole compressed input in memory, output into the caller's buffer in
 // pieces of any size.
@@ -135,6 +153,7 @@ struct RawSource {  // decompressed byte stream of a plain or gzip (multi-member
 
 struct MateTextReader {  // cuts the byte stream of one mate into batches of whole records
     RawSource src;
+    RecordCut rc;
     std::vector<uint8_t> carry;  // bytes behind the last cut
     size_t carry_pos = 0;
     bool eof = false;
@@ -154,6 +173,7 @@ struct MateTextReader {  // cuts the byte stream of one mate into batches of who
     uint64_t gz_off = 0;         // file offset of the next member
     int next_bgzf(uint32_t max_reads, PinnedBuf& buf, uint64_t* bytes, uint32_t* n_reads);
     int finish_at_eof(PinnedBuf& buf, size_t pos, uint64_t lines, uint64_t* bytes, uint32_t* n_reads);
+    int finish_fasta_at_eof(PinnedBuf& buf, size_t pos, uint64_t* bytes, uint32_t* n_reads);
 };
 
 int parse_records(const uint8_t* text, size_t n_bytes, bool at_eof, uint32_t max_reads, MateSoA& out, size_t* consumed,

@@ -450,7 +450,8 @@ __global__ void __launch_bounds__(1024) k_scan(uint32_t nblk, const uint32_t* __
 // DRAM traffic: partially written sectors were filled from and evicted to HBM).  All loads of a record are
 // issued before its first store; no shared-memory staging and no barrier in the copy loop.
 // Every source byte is read once and every output byte written once.
-// The reverse-complementing single-end sink takes a bytewise path.
+// The reverse-complementing single-end sink takes a bytewise path, and so does k_emit<true>, which writes FASTA
+// records (">name\nseq\n", CSQ_PLAN_FASTA).
 struct EmitRec {
     uint8_t* out;        // where the record goes
     uint32_t nm;         // id bytes: offset into the mate's name pool
@@ -466,9 +467,10 @@ struct EmitSrc {  // global pointers of one record
 
 constexpr int EMIT_UNROLL = 4;
 
+template <bool FASTA = false>
 __device__ __forceinline__ uint8_t emit_byte(const EmitRec& R, const EmitSrc& S, uint32_t p, uint32_t e_name, uint32_t e_umi,
                                              uint32_t e_seq, uint32_t e_qual, bool revcomp) {
-    if (p < e_name) return p == 0 ? (uint8_t)'@' : S.nm[p - 1];
+    if (p < e_name) return p == 0 ? (uint8_t)(FASTA ? '>' : '@') : S.nm[p - 1];
     if (p < e_umi) {
         uint32_t x = p - e_name;
         if (x == 0) return (uint8_t)'_';
@@ -480,6 +482,7 @@ __device__ __forceinline__ uint8_t emit_byte(const EmitRec& R, const EmitSrc& S,
         const uint32_t x = p - e_umi - 1;
         return revcomp ? complement_base(S.sq[R.b - 1 - x]) : S.sq[R.a + x];
     }
+    if (FASTA) return (uint8_t)'\n';
     if (p < e_seq + 3) return (p - e_seq == 1) ? (uint8_t)'+' : (uint8_t)'\n';
     if (p < e_qual) {
         const uint32_t x = p - e_seq - 3;
@@ -495,6 +498,7 @@ __device__ __forceinline__ void word_split(const uint8_t* dst, uint32_t len, uin
     nw = (len - head) >> 2;
 }
 
+template <bool FASTA>
 __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_emit(const __grid_constant__ EmitParams E) {
     const PairParams& P = E.pp;
     __shared__ EmitRec recs[2][CSQ_PAIR_BLOCK];
@@ -520,7 +524,7 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_emit(const __grid_constant__
         st[0] = load_state(P.md[0].state + idx);
         st[1] = paired ? load_state(P.md[1].state + idx) : st[0];
         for (int mt = 0; mt < n_mates; mt++) {
-            shape[mt] = record_shape(P, st[mt], st[0], st[1]);
+            shape[mt] = record_shape<FASTA>(P, st[mt], st[0], st[1]);
             len[mt] = shape[mt].total;
         }
     }
@@ -584,20 +588,21 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_emit(const __grid_constant__
             const uint32_t seq_len = (uint32_t)R.b - (uint32_t)R.a;
             const uint32_t e_umi = 1u + R.id_len + R.umi_len;
             uint8_t* __restrict__ out = R.out;
-            if (revcomp) {
+            if (FASTA || revcomp) {
                 EmitSrc S;
                 S.nm = md.name + R.nm;
                 S.sq = md.seq + R.sq;
                 S.ql = md.qual + R.ql;
                 S.pa = (poolA ? poolA : md.seq) + R.pa;
                 S.pb = (poolB ? poolB : md.seq) + R.pb;
-                const uint32_t e_name = 1u + R.id_len, e_seq = e_umi + 1 + seq_len, e_qual = e_seq + 3 + seq_len, total = e_qual + 1;
+                const uint32_t e_name = 1u + R.id_len, e_seq = e_umi + 1 + seq_len, e_qual = e_seq + 3 + seq_len;
+                const uint32_t total = FASTA ? e_seq + 1 : e_qual + 1;
                 for (uint32_t p0 = sl; p0 < total; p0 += G * EMIT_UNROLL) {
                     uint8_t ch[EMIT_UNROLL];
 #pragma unroll
                     for (int u = 0; u < EMIT_UNROLL; u++) {
                         const uint32_t p = p0 + G * u;
-                        ch[u] = p < total ? emit_byte(R, S, p, e_name, e_umi, e_seq, e_qual, true) : (uint8_t)0;
+                        ch[u] = p < total ? emit_byte<FASTA>(R, S, p, e_name, e_umi, e_seq, e_qual, FASTA ? revcomp : true) : (uint8_t)0;
                     }
 #pragma unroll
                     for (int u = 0; u < EMIT_UNROLL; u++) {
@@ -960,10 +965,13 @@ cudaError_t csq_launch_scan(uint32_t nblk, const uint32_t* block_tot, const uint
     return cudaGetLastError();
 }
 
-cudaError_t csq_launch_emit(const EmitParams& p, cudaStream_t stream) {
+cudaError_t csq_launch_emit(const EmitParams& p, bool fasta, cudaStream_t stream) {
     if (p.pp.n == 0) return cudaSuccess;
     const dim3 grid((p.pp.n + CSQ_PAIR_BLOCK - 1) / CSQ_PAIR_BLOCK), block(CSQ_PAIR_BLOCK);
-    k_emit<<<grid, block, 0, stream>>>(p);
+    if (fasta)
+        k_emit<true><<<grid, block, 0, stream>>>(p);
+    else
+        k_emit<false><<<grid, block, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

@@ -17,6 +17,20 @@
 // nothing is copied into a packed layout.  Bound: HBM - the text is read once (plus 1/8 of it written and read
 // back as masks and 16 bytes of line-end offsets per record written and read).  A malformed record is reported
 // as the smallest (record, kind) key through `perr`, in the order dnaio would meet the problems.
+//
+// FASTA text (CSQ_PLAN_FASTA) takes its own kernels, as transcode.fasta_to_fastq reads it:
+//   k_fa_count     reads the text once: a record-start bit mask per 16-byte chunk ('>' as the first byte of a line)
+//                  and record starts per tile; k_tile_scan and k_nl_index then turn the masks into hdr[r] = offset of
+//                  the r-th record start, exactly as they do for line ends
+//   k_fa_records   thread per record: header = the rest of the '>' line without trailing '\r'; every following line up
+//                  to the next record start is stripped of ASCII whitespace and the pieces are joined.  A sequence on
+//                  one line (the common unwrapped case, also with CRLF, blank lines or blanks around it) stays
+//                  where it is in the text; a wrapped one is marked for the pool.  Text in front of the first header
+//                  that is not blank, a different number of headers than the host counted and the read-length limit
+//                  are reported through `perr`
+//   k_tile_scan    (again) exclusive scan of the 16-byte-padded lengths of the wrapped records = their pool offsets
+//   k_fa_compact   thread per wrapped record: its stripped lines, joined, into the pool behind the text
+// Qualities are a constant buffer of 'I' bytes (qual_off the same for every record).
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -251,6 +265,174 @@ __global__ void __launch_bounds__(256) k_records(const ParseParams P) {
 }
 
 
+// ---- FASTA ----
+constexpr uint32_t FA_MULTI = 0x80000000u;  // seq_len bit between k_fa_records and k_fa_compact: sequence spans lines
+
+// bit i set <=> byte i of the 16 equals the byte replicated in kc (< 0x80)
+__device__ __forceinline__ uint32_t eq_mask16(uint4 v, uint32_t kc, const ByteConsts& k) {
+    const uint32_t M = 0x00204081u;
+    const uint32_t n0 = (eq_marks(v.x, kc, k) * M) >> 28, n1 = (eq_marks(v.y, kc, k) * M) >> 24;
+    const uint32_t n2 = (eq_marks(v.z, kc, k) * M) >> 20, n3 = (eq_marks(v.w, kc, k) * M) >> 16;
+    return n0 | (n1 & 0xF0u) | (n2 & 0xF00u) | (n3 & 0xF000u);
+}
+__device__ __forceinline__ uint32_t collapse4(uint32_t m) {  // bit 0 of every byte -> bits 0..3
+    return (((m & 0x01010101u) * 0x00204081u) >> 21) & 0xFu;
+}
+// bit i set <=> byte i is ASCII whitespace as bytes.strip() sees it: ' ', '\t', '\n', '\v', '\f', '\r'
+__device__ __forceinline__ uint32_t ws_mask16(uint4 v) {
+    auto nib = [](uint32_t w) { return collapse4(__vcmpeq4(w, 0x20202020u) | (__vcmpgeu4(w, 0x09090909u) & __vcmpleu4(w, 0x0D0D0D0Du))); };
+    return nib(v.x) | (nib(v.y) << 4) | (nib(v.z) << 8) | (nib(v.w) << 12);
+}
+__device__ __forceinline__ uint32_t nl_bits16(uint4 v) {
+    auto nib = [](uint32_t w) { return collapse4(__vcmpeq4(w, 0x0A0A0A0Au)); };
+    return nib(v.x) | (nib(v.y) << 4) | (nib(v.z) << 8) | (nib(v.w) << 12);
+}
+// bits of the 16-byte chunk at c that lie inside [b, e)
+__device__ __forceinline__ uint32_t range_bits16(uint32_t c, uint32_t b, uint32_t e) {
+    uint32_t valid = 0xFFFFu;
+    if (c < b) valid &= 0xFFFFu << (b - c);
+    if (e - c < 16u) valid &= (1u << (e - c)) - 1u;
+    return valid;
+}
+
+// Calls f(s, t) for the stripped content [s, t) of every line in [b, e) that is not blank (the last line may lack its
+// line end).  The text is 16-byte aligned and zero padded.
+template <class F>
+__device__ __forceinline__ void for_each_content(const uint8_t* __restrict__ text, uint32_t b, uint32_t e, F f) {
+    int64_t first = -1;  // first and last non-blank byte of the current line
+    uint32_t last = 0;
+    for (uint32_t c = b & ~15u; c < e; c += 16) {
+        const uint4 v = *reinterpret_cast<const uint4*>(text + c);
+        const uint32_t valid = range_bits16(c, b, e);
+        uint32_t nl = nl_bits16(v) & valid, cont = ~ws_mask16(v) & valid;
+        for (;;) {
+            const uint32_t bit = nl & (0u - nl);            // the next line end (0: none in this chunk)
+            const uint32_t seg = bit ? bit - 1u : 0xFFFFu;  // the bytes in front of it
+            const uint32_t cs = cont & seg;
+            if (cs) {
+                if (first < 0) first = c + (uint32_t)(__ffs(cs) - 1);
+                last = c + 31u - (uint32_t)__clz(cs);
+            }
+            if (!bit) break;
+            if (first >= 0) f((uint32_t)first, last + 1u);
+            first = -1;
+            cont &= ~(seg | bit);
+            nl &= ~bit;
+        }
+    }
+    if (first >= 0) f((uint32_t)first, last + 1u);
+}
+
+// Pass 1: record starts per 16-byte chunk ('>' behind a '\n', or at offset 0) and per tile.
+__global__ void __launch_bounds__(TILE_THREADS) k_fa_count(const uint8_t* __restrict__ text, uint64_t bytes,
+                                                           uint16_t* __restrict__ masks, uint32_t* __restrict__ tile_cnt) {
+    __shared__ uint32_t wsum[TILE_THREADS / 32];
+    const uint64_t tile_off = (uint64_t)blockIdx.x * TILE_BYTES;
+    uint32_t c = 0;
+    const ByteConsts k = byte_consts();
+    uint32_t kgt;
+    asm volatile("mov.b32 %0, 0x3E3E3E3E;" : "=r"(kgt));
+#pragma unroll 4
+    for (int i = 0; i < TILE_CHUNKS / TILE_THREADS; i++) {
+        const uint32_t chunk = i * TILE_THREADS + threadIdx.x;
+        const uint64_t off = tile_off + 16ull * chunk;
+        uint32_t m = 0;
+        if (off < bytes) {
+            const uint4 v = *reinterpret_cast<const uint4*>(text + off);
+            const bool line_start = off == 0 || text[off - 1] == '\n';
+            m = eq_mask16(v, kgt, k) & (((eq_mask16(v, k.k0a, k) << 1) | (line_start ? 1u : 0u)) & 0xFFFFu);
+        }
+        masks[(size_t)blockIdx.x * TILE_CHUNKS + chunk] = (uint16_t)m;
+        c += __popc(m);
+    }
+    c = __reduce_add_sync(0xffffffffu, c);
+    if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint32_t t = 0;
+#pragma unroll
+        for (int w = 0; w < TILE_THREADS / 32; w++) t += wsum[w];
+        tile_cnt[blockIdx.x] = t;
+    }
+}
+
+// kinds of a malformed FASTA batch (same key as the FASTQ kinds; 4 = PERR_LIMIT, 5 = PERR_COUNT, 7 = header limit)
+enum { PERR_FA_PREAMBLE = 1 };
+
+__global__ void __launch_bounds__(256) k_fa_records(const FastaParams F) {
+    const ParseParams& P = F.p;
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool count_ok = P.nl_total[0] == P.n;
+    if (i == 0 && !count_ok) report(P.perr, 0, PERR_COUNT);
+    if (i >= P.n) return;
+    if (!count_ok) {  // hdr[] is not fully defined: every record becomes an empty one, the host rejects the batch
+        P.name_off[i] = P.name_end[i] = P.seq_off[i] = P.seq_len[i] = 0;
+        P.qual_off[i] = F.qual0;
+        F.pad_len[i] = 0;
+        return;
+    }
+    const uint8_t* __restrict__ t = P.text;
+    const uint32_t h = P.nl[i], e = i + 1 < P.n ? P.nl[i + 1] : (uint32_t)P.bytes;
+    if (i == 0 && h > 0) {  // only blank lines may stand in front of the first header
+        bool blank = true;
+        for (uint32_t c = 0; c < h && blank; c += 16) {
+            const uint4 v = *reinterpret_cast<const uint4*>(t + c);
+            blank = (~ws_mask16(v) & range_bits16(c, 0, h)) == 0;
+        }
+        if (!blank) report(P.perr, 0, PERR_FA_PREAMBLE);
+    }
+    // the header line ends at the first '\n' behind the '>'
+    uint32_t he = e;
+    for (uint32_t c = (h + 1) & ~15u; c < e; c += 16) {
+        const uint32_t m = nl_bits16(*reinterpret_cast<const uint4*>(t + c)) & range_bits16(c, h + 1, e);
+        if (m) {
+            he = c + (uint32_t)(__ffs(m) - 1);
+            break;
+        }
+    }
+    uint32_t ne = he;
+    while (ne > h + 1 && t[ne - 1] == '\r') ne--;
+    const uint32_t body = min(he + 1, e);
+    uint32_t lines = 0, len = 0, s0 = body;
+    for_each_content(t, body, e, [&](uint32_t s, uint32_t x) {
+        if (lines == 0) s0 = s;
+        len += x - s;
+        lines++;
+    });
+    const bool ok = len <= CSQ_MAX_READ_LEN;
+    if (!ok) report(P.perr, i, PERR_LIMIT);
+    P.name_off[i] = h + 1;
+    P.name_end[i] = ne;
+    P.qual_off[i] = F.qual0;
+    const bool multi = ok && lines > 1;
+    P.seq_off[i] = multi ? body : s0;  // wrapped: where k_fa_compact starts looking
+    P.seq_len[i] = ok ? (multi ? (len | FA_MULTI) : len) : 0u;
+    F.pad_len[i] = multi ? (len + 15u) & ~15u : 0u;
+}
+
+__global__ void __launch_bounds__(256) k_fa_compact(const FastaParams F) {
+    const ParseParams& P = F.p;
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i == 0) {  // readable, defined bytes behind the last pool record for the 16-byte fetches
+        uint4* z = reinterpret_cast<uint4*>(F.pool + F.pool_total[0]);
+        for (int q = 0; q < 4; q++) z[q] = make_uint4(0, 0, 0, 0);
+    }
+    if (i >= P.n) return;
+    const uint32_t sl = P.seq_len[i];
+    if (!(sl & FA_MULTI)) return;
+    const uint32_t len = sl & ~FA_MULTI, off = F.pad_len[i];
+    const uint32_t e = i + 1 < P.n ? P.nl[i + 1] : (uint32_t)P.bytes;
+    uint8_t* __restrict__ dst = F.pool + off;
+    const uint8_t* __restrict__ t = P.text;
+    uint32_t w = 0;
+    for_each_content(t, P.seq_off[i], e, [&](uint32_t s, uint32_t x) {
+        for (uint32_t y = s; y < x; y++) dst[w++] = t[y];
+    });
+    for (; w & 15u; w++) dst[w] = 0;
+    P.seq_off[i] = F.pool0 + off;
+    P.seq_len[i] = len;
+}
+
 }  // namespace
 
 uint32_t csq_parse_tiles(uint64_t bytes) { return (uint32_t)((bytes + TILE_BYTES - 1) / TILE_BYTES); }
@@ -279,3 +461,27 @@ cudaError_t csq_launch_parse(const ParseParams& p, void* tile_buf, uint16_t* mas
     k_records<<<(p.n + 255) / 256 + (p.n == 0 ? 1 : 0), 256, 0, stream>>>(p);
     return cudaGetLastError();
 }
+
+// FASTA: k_fa_count, k_tile_scan, k_nl_index (not for an empty text), k_fa_records, k_tile_scan, k_fa_compact (not
+// for an empty batch).
+cudaError_t csq_launch_parse_fasta(const FastaParams& f, void* tile_buf, uint16_t* masks, cudaStream_t stream) {
+    const ParseParams& p = f.p;
+    const uint32_t tiles = csq_parse_tiles(p.bytes);
+    uint32_t* tile_cnt = (uint32_t*)tile_buf;
+    if (tiles) {
+        k_fa_count<<<tiles, TILE_THREADS, 0, stream>>>(p.text, p.bytes, masks, tile_cnt);
+        k_tile_scan<<<1, 1024, 0, stream>>>(tiles, tile_cnt, p.nl_total);
+        k_nl_index<<<tiles, TILE_THREADS, 0, stream>>>(masks, tile_cnt, p.nl, p.n, 0u, nullptr);
+    } else {
+        cudaError_t e = cudaMemsetAsync(p.nl_total, 0, 4, stream);
+        if (e != cudaSuccess) return e;
+    }
+    k_fa_records<<<(p.n + 255) / 256 + (p.n == 0 ? 1 : 0), 256, 0, stream>>>(f);
+    if (p.n) {
+        k_tile_scan<<<1, 1024, 0, stream>>>(p.n, f.pad_len, f.pool_total);
+        k_fa_compact<<<(p.n + 255) / 256, 256, 0, stream>>>(f);
+    }
+    return cudaGetLastError();
+}
+
+uint32_t csq_parse_fasta_launches(uint64_t bytes, uint32_t n) { return (csq_parse_tiles(bytes) ? 3u : 0u) + 1u + (n ? 2u : 0u); }

@@ -41,7 +41,7 @@
 void csq_set_error(const char* msg);
 struct csq_text_reader;
 int csq_text_reader_next_into(csq_text_reader* r, csqio::PinnedBuf* bufs, uint32_t max_reads, csq_batch_text* in);
-extern "C" int csq_text_reader_open(const char* path1, const char* path2, csq_text_reader** out);
+extern "C" int csq_text_reader_open_flags(const char* path1, const char* path2, uint32_t plan_flags, csq_text_reader** out);
 extern "C" void csq_text_reader_close(csq_text_reader* r);
 
 namespace {
@@ -294,6 +294,7 @@ struct PlainCutter {
     uint64_t records_done = 0;
     int threads = 2;
     std::string name;
+    csqio::RecordCut rc;
     // -> 0 ok (len == 0 and n == 0 at the end of the file), else error code
     int next(uint32_t max_reads, uint64_t* start, uint64_t* len, uint32_t* n, bool* append_nl) {
         *start = off;
@@ -301,7 +302,7 @@ struct PlainCutter {
         *n = 0;
         *append_nl = false;
         if (off >= f->size) return 0;
-        const uint64_t target = 4ull * max_reads;
+        const uint64_t target = rc.target(max_reads);
         const uint8_t* base = f->map + off;
         const uint64_t left = f->size - off;
         uint64_t pos = 0, lines = 0;
@@ -316,7 +317,7 @@ struct PlainCutter {
             const uint64_t per = (round + (uint64_t)nt - 1) / (uint64_t)nt;
             auto work = [&](int t) {
                 const uint64_t b = pos + (uint64_t)t * per, e = std::min(pos + round, b + per);
-                cnt[(size_t)t] = e > b ? csqio::count_newlines(base + b, (size_t)(e - b)) : 0;
+                cnt[(size_t)t] = e > b ? rc.count(base + b, (size_t)(e - b), b ? base[b - 1] : (uint8_t)'\n') : 0;
             };
             std::vector<std::thread> helpers;
             for (int t = 1; t < nt; t++) helpers.emplace_back(work, t);
@@ -325,7 +326,7 @@ struct PlainCutter {
             for (int t = 0; t < nt; t++) {
                 const uint64_t b = pos + (uint64_t)t * per, e = std::min(pos + round, b + per);
                 if (lines + cnt[(size_t)t] >= target) {
-                    const uint64_t rel = csqio::after_kth_newline(base + b, (size_t)(e - b), target - lines);
+                    const uint64_t rel = rc.cut(base + b, (size_t)(e - b), target - lines, b ? base[b - 1] : (uint8_t)'\n');
                     const uint64_t cut = b + rel;
                     *len = cut;
                     *n = max_reads;
@@ -342,6 +343,21 @@ struct PlainCutter {
         // the rest of the file holds fewer than max_reads records: dnaio accepts a missing final line end and blank
         // lines behind the last record
         uint64_t end = left;
+        if (rc.fasta) {  // every record start left is a record of the batch; text without one must be blank
+            if (lines == 0) {
+                for (uint64_t i = 0; i < end; i++)
+                    if (base[i] != ' ' && (base[i] < 9 || base[i] > 13))
+                        return csqio::io_fail(CSQ_ERR_FORMAT, "%s: FASTA input does not start with a '>' header (line %llu)", name.c_str(),
+                                              (unsigned long long)(csqio::count_newlines(base, (size_t)i) + 1));
+                end = 0;
+            }
+            *append_nl = end && base[end - 1] != '\n';
+            *len = end;
+            *n = (uint32_t)lines;
+            records_done += lines;
+            off = f->size;
+            return 0;
+        }
         if (end && base[end - 1] != '\n') {
             *append_nl = true;
             lines++;
@@ -420,7 +436,15 @@ extern "C" int csq_run_files(const csq_op* ops_r1, int n1, const csq_op* ops_r2,
     }
     for (int m = 0; m < n_mates; m++)
         if (inf[m].regular && inf[m].size == 0) all_plain = all_bgzf = false;  // empty files: the serial reader knows what to do
+    // FASTA never takes mode 1: the line ends per member do not tell where FASTA records start
+    const bool fasta = (plan_flags & CSQ_PLAN_FASTA) != 0;
+    if (fasta) all_bgzf = false;
     const int mode = all_plain ? 0 : all_bgzf ? 1 : 2;  // 0 plain ranges, 1 BGZF member runs, 2 serial text reader
+    const csqio::RecordCut record_cut{fasta};
+    // records in a sample of text (a FASTA record has any number of lines)
+    auto sample_records = [&](const uint8_t* t, size_t n) -> double {
+        return fasta ? (double)csqio::count_fasta_records(t, n, '\n') : (double)csqio::count_newlines(t, n) / 4.0;
+    };
     const uint32_t batch_reads = files->batch_reads ? files->batch_reads : (mode == 2 ? (1u << 16) : (1u << 18));
 
     // plans: one thread per GPU creates its context and plan (0.3 - 0.5 s each when done one after the other)
@@ -453,7 +477,7 @@ extern "C" int csq_run_files(const csq_op* ops_r1, int n1, const csq_op* ops_r2,
 
     csq_text_reader* reader = nullptr;
     if (mode == 2) {
-        int rc = csq_text_reader_open(files->in[0], files->in[1], &reader);
+        int rc = csq_text_reader_open_flags(files->in[0], files->in[1], plan_flags, &reader);
         if (rc) {
             destroy_plans();
             return rc;
@@ -502,7 +526,9 @@ extern "C" int csq_run_files(const csq_op* ops_r1, int n1, const csq_op* ops_r2,
         for (int m = 0; m < 2; m++) {
             uint64_t full = 64;
             if (m < n_mates) {
-                full = text[m] + 64ull * n + 4096;  // renaming can only shorten a record, bar "_" + UMI
+                // renaming can only shorten a record, bar "_" + UMI; a FASTA record comes out with at most one line end
+                // more than it had (">a\n" in front of the next header: ">a\n\n")
+                full = text[m] + 64ull * n + 4096;
                 if (device_gzip) full = full / 2;   // the packed size is reported when this guess is too small
             }
             for (int d = 0; d < CSQ_N_DEST; d++) want[d][m] = m >= n_mates ? 64 : d == CSQ_DEST_TRIMMED ? full : full / 8 + 4096;
@@ -541,12 +567,12 @@ extern "C" int csq_run_files(const csq_op* ops_r1, int n1, const csq_op* ops_r2,
                     memcpy(text.data(), inf[m].map, (size_t)got);
                     total_text = inf[m].size;
                 }
-                const uint64_t lines = got > 0 ? csqio::count_newlines(text.data(), (size_t)got) : 0;
-                if (lines >= 4) bpr = (double)got / ((double)lines / 4.0);
+                const double recs = got > 0 ? sample_records(text.data(), (size_t)got) : 0;
+                if (recs >= 1) bpr = (double)got / recs;
             } else if (mode == 0) {
                 const size_t sample = (size_t)std::min<uint64_t>(inf[m].size, 4u << 20);
-                const uint64_t lines = csqio::count_newlines(inf[m].map, sample);
-                if (lines >= 4) bpr = (double)sample / ((double)lines / 4.0);
+                const double recs = sample_records(inf[m].map, sample);
+                if (recs >= 1) bpr = (double)sample / recs;
                 total_text = inf[m].size;
             } else {
                 for (size_t i = 0; i < inf[m].isize.size() && bpr == 0; i++) {
@@ -865,6 +891,7 @@ extern "C" int csq_run_files(const csq_op* ops_r1, int n1, const csq_op* ops_r2,
                 cut[m].f = &inf[m];
                 cut[m].name = files->in[m];
                 cut[m].threads = std::max(1, std::min(6, n_threads / (2 * n_mates)));
+                cut[m].rc = record_cut;
             }
             while (!sh.stop && free_q.pop(j)) {
                 uint32_t n[2] = {0, 0};

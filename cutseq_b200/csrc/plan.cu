@@ -96,6 +96,12 @@ struct Slot {
     uint64_t text_bytes[2] = {0, 0};
     uint64_t first_record = 0;
     bool text_mode = false;
+    // CSQ_PLAN_FASTA: the plan's buffer of 'I' qualities, the padded lengths / pool offsets of wrapped records, and the
+    // batch text of csq_submit_text (caller memory, alive until csq_wait) for the file lines of error texts
+    const uint8_t* fasta_qual = nullptr;
+    DevBuf fa_pad[2];
+    const uint8_t* host_text[2] = {nullptr, nullptr};
+    uint64_t host_bytes[2] = {0, 0};
     unsigned long long* totals_host = nullptr;  // pinned: 12 totals + 2 error flags + 2 parse-error keys
     uint32_t n = 0;
     int n_mates = 0;
@@ -118,6 +124,7 @@ struct csq_plan {
     int* error_flag = nullptr;
     uint32_t* gz_tables = nullptr;           // device: CRC-32 byte table [256] | fold operators [GZ_THREADS]
     uint32_t* crc_check_tables = nullptr;    // device: tables of the member CRC check behind the device inflate [768]
+    uint8_t* fasta_qual = nullptr;           // device, CSQ_PLAN_FASTA: CSQ_FASTA_QUAL_BYTES of 'I'
     uint64_t launches = 0;
 };
 
@@ -302,6 +309,7 @@ MateDev mate_dev(Slot& s, int m) {
     d.state = (ReadState*)s.state[m].p;
     if (s.text_mode) {
         d.seq = d.qual = d.name = (const uint8_t*)s.text[m].p + TEXT_FRONT_PAD;
+        if (s.fasta_qual) d.qual = s.fasta_qual;  // FASTA: every read has qualities 'I', as the FASTQ the pump made had
         d.qual_off = (const uint32_t*)s.qual_off[m].p;
         d.name_end = (const uint32_t*)s.name_end[m].p;
     } else {
@@ -369,7 +377,12 @@ int ensure_text_index(csq_plan* plan, Slot& s, int m, uint32_t n, uint64_t bytes
     return 0;
 }
 
-// FASTQ text of a batch -> device, as it is; the record index is built by the parse kernels in enqueue_front
+// FASTA batches: the pool of joined wrapped sequences sits behind the text in the same buffer, at this offset from the
+// text; it takes at most the text's bytes plus 16 per record (16-byte-padded slots) plus the zeroed 64 bytes behind it
+uint64_t fasta_pool0(uint64_t bytes) { return ((bytes + 63) & ~(uint64_t)63) + 128; }
+uint64_t fasta_pool_bytes(uint64_t bytes, uint32_t n) { return ((bytes + 63) & ~(uint64_t)63) + 16ull * n + 128; }
+
+// FASTQ (or FASTA) text of a batch -> device, as it is; the record index is built by the parse kernels in enqueue_front
 int upload_text(csq_plan* plan, Slot& s, const csq_batch_text* in) {
     const uint32_t n = in->n_reads;
     s.n = n;
@@ -383,8 +396,10 @@ int upload_text(csq_plan* plan, Slot& s, const csq_batch_text* in) {
         const uint64_t bytes = in->mate[m].bytes;
         s.text_bytes[m] = bytes;
         const size_t padded = (size_t)((bytes + 63) & ~(uint64_t)63);
-        if ((rc = s.text[m].ensure(TEXT_FRONT_PAD + padded + 128))) return rc;
+        const size_t pool = s.fasta_qual ? (size_t)fasta_pool_bytes(bytes, n) : 0;
+        if ((rc = s.text[m].ensure(TEXT_FRONT_PAD + padded + 128 + pool))) return rc;
         if ((rc = ensure_text_index(plan, s, m, n, bytes))) return rc;
+        if (s.fasta_qual && (rc = s.fa_pad[m].ensure((size_t)n * 4 + 64))) return rc;
         uint8_t* base = (uint8_t*)s.text[m].p;
         CUDA_TRY(cudaMemsetAsync(base, 0, TEXT_FRONT_PAD, s.stream));
         // zero padding behind the text: never a line end, and readable by the 128-bit walks
@@ -392,6 +407,7 @@ int upload_text(csq_plan* plan, Slot& s, const csq_batch_text* in) {
         if (bytes) CUDA_TRY(cudaMemcpyAsync(base + TEXT_FRONT_PAD, in->mate[m].text, bytes, cudaMemcpyHostToDevice, s.stream));
     }
     if ((rc = s.parse_misc.ensure(64))) return rc;
+    s.host_text[0] = s.host_text[1] = nullptr;
     return ensure_common(plan, s, n);
 }
 
@@ -534,7 +550,7 @@ PairParams pair_params(csq_plan* plan, Slot& s) {
 int enqueue_mate(csq_plan* plan, Slot& s, int m, KernelTimer* kt, cudaStream_t st) {
     const uint32_t n = s.n;
     if (s.text_mode) {
-        // FASTQ text -> record index (parse.cu); nl_total[m] at parse_misc + 4 m, perr[m] at parse_misc + 16 + 8 m
+        // FASTQ / FASTA text -> record index (parse.cu); nl_total[m] at parse_misc + 4 m, perr[m] at parse_misc + 16 + 8 m
         ParseParams pp;
         pp.text = (const uint8_t*)s.text[m].p + TEXT_FRONT_PAD;
         pp.bytes = s.text_bytes[m];
@@ -550,8 +566,21 @@ int enqueue_mate(csq_plan* plan, Slot& s, int m, KernelTimer* kt, cudaStream_t s
         pp.any_cr = (uint32_t*)((uint8_t*)s.parse_misc.p + 40) + m;
         pp.skip = s.bgzf_mode ? s.skip_lines[m] : 0u;
         pp.first_off = s.bgzf_mode ? (uint32_t*)((uint8_t*)s.parse_misc.p + 48) + m : nullptr;
-        CUDA_TRY(csq_launch_parse(pp, s.tiles[m].p, (uint16_t*)s.masks[m].p, st));
-        plan->launches += csq_parse_tiles(pp.bytes) ? 4 : 1;
+        if (s.fasta_qual) {
+            // FASTA: pool_total[m] at parse_misc + 56 + 4 m
+            FastaParams fp;
+            fp.p = pp;
+            fp.pool0 = (uint32_t)fasta_pool0(pp.bytes);
+            fp.pool = (uint8_t*)s.text[m].p + TEXT_FRONT_PAD + fp.pool0;
+            fp.pad_len = (uint32_t*)s.fa_pad[m].p;
+            fp.pool_total = (uint32_t*)((uint8_t*)s.parse_misc.p + 56) + m;
+            fp.qual0 = 64;
+            CUDA_TRY(csq_launch_parse_fasta(fp, s.tiles[m].p, (uint16_t*)s.masks[m].p, st));
+            plan->launches += csq_parse_fasta_launches(pp.bytes, n);
+        } else {
+            CUDA_TRY(csq_launch_parse(pp, s.tiles[m].p, (uint16_t*)s.masks[m].p, st));
+            plan->launches += csq_parse_tiles(pp.bytes) ? 4 : 1;
+        }
         if (kt) kt->mark(m == 0 ? "k_parse.r1" : "k_parse.r2");
     }
     MateProgram& mp = plan->prog[m];
@@ -618,7 +647,7 @@ int enqueue_front(csq_plan* plan, Slot& s, KernelTimer* kt, cudaStream_t st, cud
         fp[m].counters = plan->counters;
         fp[m].perr = s.text_mode ? (unsigned long long*)((uint8_t*)s.parse_misc.p + 16) + m : nullptr;
     }
-    CUDA_TRY(csq_launch_tail(fp[0], fp[1], pp, st));
+    CUDA_TRY(csq_launch_tail(fp[0], fp[1], pp, s.fasta_qual != nullptr, st));
     plan->launches += n ? 1 : 0;
     if (kt) kt->mark("k_tail");
     if (s.text_mode)  // parse errors: k_records' and k_tail's ('@' / '+' line starts)
@@ -650,10 +679,11 @@ int enqueue_emit(csq_plan* plan, Slot& s, KernelTimer* kt, cudaStream_t st) {
     for (int d = 0; d < CSQ_N_DEST; d++)
         for (int m = 0; m < 2; m++) ep.out[d][m] = (uint8_t*)s.out[d][m].p;
     // default: staged through shared memory; the direct kernels stay for A/B runs and for the reverse-complementing sink
+    const bool fasta = s.fasta_qual != nullptr;
     if ((plan->flags & CSQ_PLAN_EMIT_G16) || ep.pp.revcomp)
-        CUDA_TRY(csq_launch_emit(ep, st));
+        CUDA_TRY(csq_launch_emit(ep, fasta, st));
     else
-        CUDA_TRY(csq_launch_emit_stage(ep, st));
+        CUDA_TRY(csq_launch_emit_stage(ep, fasta, st));
     plan->launches += s.n ? 1 : 0;
     if (kt) kt->mark("k_emit");
     return 0;
@@ -707,6 +737,44 @@ int enqueue_gz(csq_plan* plan, Slot& s, KernelTimer* kt, cudaStream_t st) {
     return 0;
 }
 
+// Line (1-based, within the batch) of the header of record `rec` of a FASTA batch, or of the first line in front of
+// the first header that is not blank (rec = UINT64_MAX); 0 when the batch text is not at hand (csq_upload_text).
+uint64_t fasta_batch_line(const Slot& s, int m, uint64_t rec) {
+    const uint8_t* t = s.host_text[m];
+    const uint64_t n = s.host_bytes[m];
+    if (!t) return 0;
+    uint64_t off = 0;
+    if (rec == UINT64_MAX) {
+        while (off < n && (t[off] == ' ' || (t[off] >= 9 && t[off] <= 13))) off++;
+    } else {
+        off = csq_after_kth_fasta_record(t, n, rec);
+        if (off == UINT64_MAX) return 0;
+    }
+    return csq_count_newlines(t, off) + 1;
+}
+
+// FASTA format errors found by k_fa_records and k_tail.  Lines are file lines in the first batch of a file; further on
+// the batch's first record is named as well.
+int check_fasta_error(Slot& s, int m, unsigned long long key) {
+    const unsigned long long rec = key >> 3;
+    const int kind = (int)(key & 7);
+    char where[160];
+    const uint64_t line = fasta_batch_line(s, m, kind == 1 ? UINT64_MAX : rec);
+    if (s.first_record == 0 && line)
+        snprintf(where, sizeof(where), "line %llu", (unsigned long long)line);
+    else if (line)
+        snprintf(where, sizeof(where), "line %llu of the batch that starts with record %llu", (unsigned long long)line,
+                 (unsigned long long)s.first_record + 1);
+    else
+        snprintf(where, sizeof(where), "record %llu", (unsigned long long)(s.first_record + rec + 1));
+    switch (kind) {
+        case 1: return fail(CSQ_ERR_FORMAT, "input file %d: FASTA input does not start with a '>' header (%s)", m + 1, where);
+        case 4: return fail(CSQ_ERR_LIMIT, "input file %d: read at %s exceeds the supported %d bases", m + 1, where, CSQ_MAX_READ_LEN);
+        case 7: return fail(CSQ_ERR_LIMIT, "input file %d: header at %s exceeds the supported 65535 bytes", m + 1, where);
+        default: return fail(CSQ_ERR_FORMAT, "input file %d: the batch does not hold %u FASTA records", m + 1, s.n);
+    }
+}
+
 // FASTQ format errors found by k_records, worded like dnaio's FastqFormatError
 int check_parse_error(Slot& s) {
     if (!s.text_mode) return 0;
@@ -718,6 +786,7 @@ int check_parse_error(Slot& s) {
     for (int m = 0; m < s.n_mates; m++) {
         const unsigned long long key = s.totals_host[14 + m];
         if (key == ~0ULL) continue;
+        if (s.fasta_qual) return check_fasta_error(s, m, key);
         const unsigned long long rec = key >> 3, line = 4 * (s.first_record + rec);
         switch ((int)(key & 7)) {
             case 1: return fail(CSQ_ERR_FORMAT, "input file %d: line %llu is expected to start with '@'", m + 1, line + 1);
@@ -823,8 +892,13 @@ int csq_plan_create(const csq_op* ops_r1, int n1, const csq_op* ops_r2, int n2, 
         e = cudaMalloc((void**)&plan->gz_tables, tab.size() * 4);
         if (e == cudaSuccess) e = cudaMemcpy(plan->gz_tables, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice);
     }
+    if (e == cudaSuccess && (flags & CSQ_PLAN_FASTA)) {
+        e = cudaMalloc((void**)&plan->fasta_qual, CSQ_FASTA_QUAL_BYTES);
+        if (e == cudaSuccess) e = cudaMemset(plan->fasta_qual, 'I', CSQ_FASTA_QUAL_BYTES);
+    }
     for (int i = 0; i < CSQ_N_SLOTS && e == cudaSuccess; i++) {
         Slot& s = plan->slots[i];
+        s.fasta_qual = plan->fasta_qual;
         e = cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s.stream2, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_fork, cudaEventDisableTiming);
@@ -861,6 +935,7 @@ void csq_plan_destroy(csq_plan* plan) {
         if (s.stream2) cudaStreamDestroy(s.stream2);
         for (int m = 0; m < 2; m++) {
             s.text[m].release(); s.qual_off[m].release(); s.name_end[m].release(); s.nl[m].release(); s.tiles[m].release(); s.masks[m].release();
+            s.fa_pad[m].release();
         }
         s.dest.release(); s.block_tot.release(); s.block_cnt.release(); s.block_off.release(); s.totals.release();
         for (cudaEvent_t& e : s.ev) if (e) cudaEventDestroy(e);
@@ -876,11 +951,13 @@ void csq_plan_destroy(csq_plan* plan) {
     if (plan->error_flag) cudaFree(plan->error_flag);
     if (plan->gz_tables) cudaFree(plan->gz_tables);
     if (plan->crc_check_tables) cudaFree(plan->crc_check_tables);
+    if (plan->fasta_qual) cudaFree(plan->fasta_qual);
     delete plan;
 }
 
 int csq_submit(csq_plan* plan, int slot, const csq_batch_in* in, csq_batch_out* out) {
     if (!plan || slot < 0 || slot >= CSQ_N_SLOTS || !out) return fail(CSQ_ERR_INVALID, "bad plan/slot/out");
+    if (plan->flags & CSQ_PLAN_FASTA) return fail(CSQ_ERR_INVALID, "a CSQ_PLAN_FASTA plan takes text batches only");
     int rc = validate_batch(plan, in);
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(plan->device));
@@ -904,6 +981,11 @@ static int validate_text(const csq_plan* plan, const csq_batch_text* in) {
     }
     // the look-back words of the parse kernel count line ends in 30 bits
     if ((uint64_t)in->n_reads * 4 >= (1ull << 30)) return fail(CSQ_ERR_LIMIT, "too many records in one batch (limit 2^28 - 1)");
+    // FASTA: text and pool of joined sequences share one buffer addressed by 32-bit offsets
+    if (plan->flags & CSQ_PLAN_FASTA)
+        for (int m = 0; m < plan->n_mates; m++)
+            if (fasta_pool0(in->mate[m].bytes) + fasta_pool_bytes(in->mate[m].bytes, in->n_reads) >= (1ull << 32) - 4096)
+                return fail(CSQ_ERR_LIMIT, "FASTA batch text must stay below 2 GiB");
     return 0;
 }
 
@@ -916,6 +998,10 @@ int csq_submit_text(csq_plan* plan, int slot, const csq_batch_text* in, csq_batc
     if (s.pending) return fail(CSQ_ERR_INVALID, "slot %d still has a batch in flight (call csq_wait)", slot);
     CUDA_TRY(cudaEventRecord(s.ev[0], s.stream));
     if ((rc = upload_text(plan, s, in))) return rc;
+    for (int m = 0; m < plan->n_mates; m++) {
+        s.host_text[m] = in->mate[m].text;
+        s.host_bytes[m] = in->mate[m].bytes;
+    }
     CUDA_TRY(cudaEventRecord(s.ev[1], s.stream));
     if ((rc = enqueue_front(plan, s, nullptr, s.stream, s.stream2))) return rc;
     CUDA_TRY(cudaEventRecord(s.ev[2], s.stream));
@@ -925,6 +1011,7 @@ int csq_submit_text(csq_plan* plan, int slot, const csq_batch_text* in, csq_batc
 
 int csq_submit_bgzf(csq_plan* plan, int slot, const csq_batch_bgzf* in, csq_batch_out* out) {
     if (!plan || slot < 0 || slot >= CSQ_N_SLOTS || !out || !in) return fail(CSQ_ERR_INVALID, "bad plan/slot/in/out");
+    if (plan->flags & CSQ_PLAN_FASTA) return fail(CSQ_ERR_INVALID, "a CSQ_PLAN_FASTA plan takes text batches only (BGZF batches are cut by line ends)");
     if ((int)in->n_mates != plan->n_mates) return fail(CSQ_ERR_INVALID, "batch has %u mates, plan has %d", in->n_mates, plan->n_mates);
     if ((uint64_t)in->n_reads * 4 >= (1ull << 30)) return fail(CSQ_ERR_LIMIT, "too many records in one batch (limit 2^28 - 1)");
     CUDA_TRY(cudaSetDevice(plan->device));
@@ -942,6 +1029,7 @@ int csq_submit_bgzf(csq_plan* plan, int slot, const csq_batch_bgzf* in, csq_batc
 
 int csq_bgzf_count_lines(csq_plan* plan, int slot, const csq_bgzf_in* in, uint32_t* lines) {
     if (!plan || slot < 0 || slot >= CSQ_N_SLOTS || !in || (in->n_members && !lines)) return fail(CSQ_ERR_INVALID, "bad argument");
+    if (plan->flags & CSQ_PLAN_FASTA) return fail(CSQ_ERR_INVALID, "a CSQ_PLAN_FASTA plan takes text batches only (BGZF batches are cut by line ends)");
     CUDA_TRY(cudaSetDevice(plan->device));
     Slot& s = plan->slots[slot];
     if (s.pending) return fail(CSQ_ERR_INVALID, "slot %d still has a batch in flight (call csq_wait)", slot);
@@ -1048,6 +1136,7 @@ int csq_slot_times(csq_plan* plan, int slot, float* total_ms, float* kernel_ms) 
 
 int csq_upload(csq_plan* plan, int slot, const csq_batch_in* in) {
     if (!plan || slot < 0 || slot >= CSQ_N_SLOTS) return fail(CSQ_ERR_INVALID, "bad plan/slot");
+    if (plan->flags & CSQ_PLAN_FASTA) return fail(CSQ_ERR_INVALID, "a CSQ_PLAN_FASTA plan takes text batches only");
     int rc = validate_batch(plan, in);
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(plan->device));

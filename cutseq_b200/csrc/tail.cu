@@ -8,6 +8,8 @@
 // registers between "finish" and the pair decision, the states are written once, and the header bytes that the id
 // parser fetches anyway are compared for the name check (the emitters no longer look at ids).
 // In text batches the '@' / '+' line starts of the FASTQ parser are checked here too (parse.cu, k_records).
+// k_tail<true> serves FASTA batches (CSQ_PLAN_FASTA): the '>' in front of the header and the header limit are checked,
+// there is no '+' line, and records are ">name\nseq\n".
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -47,6 +49,7 @@ struct MateTail {
 };
 
 // One mate: trailing scalar ops, quality trimming, header suffixes and id.  Returns the bases removed by QTRIM.
+template <bool FASTA>
 __device__ __forceinline__ uint32_t finish_mate(const FinishParams& P, uint32_t idx, MateTail& T) {
     const uint32_t len0 = P.md.seq_len[idx];
     ReadState st = P.first ? fresh_state(len0) : load_state(P.md.state + idx);
@@ -61,7 +64,14 @@ __device__ __forceinline__ uint32_t finish_mate(const FinishParams& P, uint32_t 
         // bases with '+'; both bytes sit in sectors this thread fetches anyway.  Records at or behind an error
         // that is already known are skipped (the host reports the smallest key).
         const unsigned long long known = *reinterpret_cast<volatile unsigned long long*>(P.perr);
-        if ((known >> 3) > (unsigned long long)idx) {
+        if (FASTA) {
+            if ((known >> 3) > (unsigned long long)idx) {
+                int bad = 0;
+                if (nm[-1] != '>') bad = 5;                                 // PERR_COUNT: not a record start
+                else if (nl > 65535) bad = 7;                               // header limit
+                if (bad) atomicMin(P.perr, ((unsigned long long)idx << 3) | (unsigned long long)bad);
+            }
+        } else if ((known >> 3) > (unsigned long long)idx) {
             const uint8_t* se = P.md.seq + P.md.seq_off[idx] + len0;  // the line end behind the bases
             int bad = 0;
             const uint8_t* pl = se + (se[0] == '\r' ? 2 : 1);         // the third line
@@ -260,6 +270,7 @@ struct TailParams {
     PairParams pp;
 };
 
+template <bool FASTA>
 __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_tail(const __grid_constant__ TailParams T) {
     const PairParams& P = T.pp;
     __shared__ unsigned int tot[8];   // bytes per (dest, mate) stream
@@ -278,10 +289,10 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_tail(const __grid_constant__
     bool bad_names = false;
     if (idx < P.n) {
         MateTail m1, m2;
-        q1 = finish_mate(T.fin[0], idx, m1);
+        q1 = finish_mate<FASTA>(T.fin[0], idx, m1);
         in1 = m1.len0;
         if (paired) {
-            q2 = finish_mate(T.fin[1], idx, m2);
+            q2 = finish_mate<FASTA>(T.fin[1], idx, m2);
             in2 = m2.len0;
             bad_names = !pair_names_ok(m1, m2, P.check_ids != 0);
         }
@@ -296,8 +307,8 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_tail(const __grid_constant__
         else
             dest = CSQ_DEST_TRIMMED;
         P.dest[idx] = (uint8_t)dest;
-        len1 = record_shape(P, s1, s1, s2).total;
-        if (paired) len2 = record_shape(P, s2, s1, s2).total;
+        len1 = record_shape<FASTA>(P, s1, s1, s2).total;
+        if (paired) len2 = record_shape<FASTA>(P, s2, s1, s2).total;
     }
     const int lane = threadIdx.x & 31;
     if (__any_sync(0xffffffffu, bad_names) && lane == 0) atomicExch(P.error_flag, (int)CSQ_ERR_PAIRING);
@@ -352,12 +363,16 @@ __global__ void __launch_bounds__(CSQ_PAIR_BLOCK) k_tail(const __grid_constant__
 
 }  // namespace
 
-cudaError_t csq_launch_tail(const FinishParams& f1, const FinishParams& f2, const PairParams& p, cudaStream_t stream) {
+cudaError_t csq_launch_tail(const FinishParams& f1, const FinishParams& f2, const PairParams& p, bool fasta, cudaStream_t stream) {
     if (p.n == 0) return cudaSuccess;
     TailParams T;
     T.fin[0] = f1;
     T.fin[1] = f2;
     T.pp = p;
-    k_tail<<<(p.n + CSQ_PAIR_BLOCK - 1) / CSQ_PAIR_BLOCK, CSQ_PAIR_BLOCK, 0, stream>>>(T);
+    const uint32_t grid = (p.n + CSQ_PAIR_BLOCK - 1) / CSQ_PAIR_BLOCK;
+    if (fasta)
+        k_tail<true><<<grid, CSQ_PAIR_BLOCK, 0, stream>>>(T);
+    else
+        k_tail<false><<<grid, CSQ_PAIR_BLOCK, 0, stream>>>(T);
     return cudaGetLastError();
 }

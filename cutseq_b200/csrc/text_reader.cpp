@@ -1,6 +1,7 @@
 // Host side of text batches: the reader only moves bytes.  It inflates (or reads) the input
 // straight into pinned memory, counts line ends to cut the stream at a record boundary
-// (4 lines per record, the same number of records for both mates) and hands the bytes to
+// (4 lines per record, the same number of records for both mates; FASTA: record starts, '>' at the
+// start of a line) and hands the bytes to
 // csq_submit_text; FASTQ parsing and validation happen on the device (parse.cu).
 // Stands where xopen + dnaio's chunked reader (read_paired_chunks) sit behind cutadapt's
 // InputPaths in the reference (run.py:434-436, 751-753).
@@ -61,6 +62,54 @@ uint64_t after_kth_newline(const uint8_t* p, size_t n, uint64_t k) {
         if (!q) return UINT64_MAX;
         i = (size_t)(q - p) + 1;
         if (--k == 0) return i;
+    }
+    return UINT64_MAX;
+}
+
+#if defined(__SSE2__)
+// bit i set <=> p[i] == c, for the 64 bytes at p
+static inline uint64_t eq_mask64(const uint8_t* p, __m128i c) {
+    const uint64_t m0 = (unsigned)_mm_movemask_epi8(_mm_cmpeq_epi8(_mm_loadu_si128((const __m128i*)p), c));
+    const uint64_t m1 = (unsigned)_mm_movemask_epi8(_mm_cmpeq_epi8(_mm_loadu_si128((const __m128i*)(p + 16)), c));
+    const uint64_t m2 = (unsigned)_mm_movemask_epi8(_mm_cmpeq_epi8(_mm_loadu_si128((const __m128i*)(p + 32)), c));
+    const uint64_t m3 = (unsigned)_mm_movemask_epi8(_mm_cmpeq_epi8(_mm_loadu_si128((const __m128i*)(p + 48)), c));
+    return m0 | (m1 << 16) | (m2 << 32) | (m3 << 48);
+}
+#endif
+
+uint64_t count_fasta_records(const uint8_t* p, size_t n, uint8_t prev) {
+    uint64_t c = 0, line_start = prev == '\n' ? 1 : 0;
+    size_t i = 0;
+#if defined(__SSE2__)
+    const __m128i gt = _mm_set1_epi8('>'), nl = _mm_set1_epi8('\n');
+    for (; i + 64 <= n; i += 64) {
+        const uint64_t g = eq_mask64(p + i, gt), l = eq_mask64(p + i, nl);
+        c += (uint64_t)__builtin_popcountll(g & ((l << 1) | line_start));
+        line_start = l >> 63;
+    }
+#endif
+    for (; i < n; i++) {
+        c += p[i] == '>' && line_start;
+        line_start = p[i] == '\n';
+    }
+    return c;
+}
+
+uint64_t kth_fasta_record(const uint8_t* p, size_t n, uint64_t k, uint8_t prev) {
+    if (k == 0) return UINT64_MAX;
+    // skip whole 4 KiB blocks by count, then walk the block that holds the k-th record start
+    size_t i = 0;
+    while (i < n) {
+        const size_t len = n - i < 4096 ? n - i : 4096;
+        const uint64_t c = count_fasta_records(p + i, len, i ? p[i - 1] : prev);
+        if (c >= k) break;
+        k -= c;
+        i += len;
+    }
+    uint8_t before = i ? p[i - 1] : prev;
+    for (; i < n; i++) {
+        if (p[i] == '>' && before == '\n' && --k == 0) return i;
+        before = p[i];
     }
     return UINT64_MAX;
 }
@@ -286,7 +335,7 @@ static size_t bgzf_member_size(const uint8_t* p, size_t n) {
 }
 
 int MateTextReader::next_bgzf(uint32_t max_reads, PinnedBuf& buf, uint64_t* bytes, uint32_t* n_reads) {
-    const uint64_t target = 4ull * max_reads;
+    const uint64_t target = rc.target(max_reads);
     *bytes = 0;
     *n_reads = 0;
     size_t pos = 0;      // bytes in buf
@@ -294,9 +343,9 @@ int MateTextReader::next_bgzf(uint32_t max_reads, PinnedBuf& buf, uint64_t* byte
     const size_t avail = carry.size() - carry_pos;
     if (avail) {  // what the previous batch left behind its cut
         const uint8_t* c = carry.data() + carry_pos;
-        const uint64_t k = count_newlines(c, avail);
+        const uint64_t k = rc.count(c, avail, '\n');
         if (k >= target) {
-            const uint64_t cut = after_kth_newline(c, avail, target);
+            const uint64_t cut = rc.cut(c, avail, target, '\n');
             if (!buf.reserve((size_t)cut + 64, 0)) return io_fail(CSQ_ERR_NOMEM, "out of host memory for a batch of %u reads", max_reads);
             memcpy(buf.p, c, (size_t)cut);
             carry_pos += (size_t)cut;
@@ -355,7 +404,7 @@ int MateTextReader::next_bgzf(uint32_t max_reads, PinnedBuf& buf, uint64_t* byte
                     mb.err = inf.error()[0] ? "corrupt BGZF member" : "BGZF member size does not match its trailer";
                     continue;
                 }
-                mb.lines = count_newlines(buf.p + mb.out_off, mb.isize);
+                mb.lines = rc.count(buf.p + mb.out_off, mb.isize, 0);  // + the record start at its edge, below
             }
         };
         int nt = read_threads;
@@ -364,11 +413,13 @@ int MateTextReader::next_bgzf(uint32_t max_reads, PinnedBuf& buf, uint64_t* byte
         for (int t = 1; t < nt; t++) helpers.emplace_back(work);
         work();
         for (auto& th : helpers) th.join();
-        for (const Member& mb : mems)
+        for (Member& mb : mems) {
             if (mb.err) return io_fail(CSQ_ERR_IO, "%s: %s", src.name.c_str(), mb.err);
+            mb.lines += rc.edge(buf.p + mb.out_off, mb.isize, mb.out_off ? buf.p[mb.out_off - 1] : '\n');
+        }
         for (const Member& mb : mems) {
             if (lines + mb.lines >= target) {
-                const uint64_t rel = after_kth_newline(buf.p + mb.out_off, mb.isize, target - lines);
+                const uint64_t rel = rc.cut(buf.p + mb.out_off, mb.isize, target - lines, mb.out_off ? buf.p[mb.out_off - 1] : '\n');
                 const size_t cut = mb.out_off + (size_t)rel;
                 carry.assign(buf.p + cut, buf.p + pos + acc);
                 hint_bytes = cut;
@@ -388,6 +439,7 @@ int MateTextReader::next_bgzf(uint32_t max_reads, PinnedBuf& buf, uint64_t* byte
 
 // End of the input: a missing final line end is accepted, and so are blank lines behind the last record (dnaio).
 int MateTextReader::finish_at_eof(PinnedBuf& buf, size_t pos, uint64_t lines, uint64_t* bytes, uint32_t* n_reads) {
+    if (rc.fasta) return finish_fasta_at_eof(buf, pos, bytes, n_reads);
     if (pos && buf.p[pos - 1] != '\n') {
         if (!buf.reserve(pos + 64, pos)) return io_fail(CSQ_ERR_NOMEM, "out of host memory");
         buf.p[pos++] = '\n';
@@ -416,12 +468,32 @@ int MateTextReader::finish_at_eof(PinnedBuf& buf, size_t pos, uint64_t lines, ui
     return 0;
 }
 
+// FASTA: every record start left is a record of the batch; a missing final line end is added.  Text without a record
+// (only possible in front of the first one) must be blank.
+int MateTextReader::finish_fasta_at_eof(PinnedBuf& buf, size_t pos, uint64_t* bytes, uint32_t* n_reads) {
+    const uint64_t n = count_fasta_records(buf.p, pos, '\n');
+    if (n == 0) {
+        for (size_t i = 0; i < pos; i++)
+            if (buf.p[i] != ' ' && (buf.p[i] < 9 || buf.p[i] > 13))
+                return io_fail(CSQ_ERR_FORMAT, "%s: FASTA input does not start with a '>' header (line %llu)", src.name.c_str(),
+                               (unsigned long long)(count_newlines(buf.p, i) + 1));
+        pos = 0;
+    } else if (buf.p[pos - 1] != '\n') {
+        if (!buf.reserve(pos + 64, pos)) return io_fail(CSQ_ERR_NOMEM, "out of host memory");
+        buf.p[pos++] = '\n';
+    }
+    *bytes = pos;
+    *n_reads = (uint32_t)n;
+    records_done += n;
+    return 0;
+}
+
 // Plain regular file: the next batch is [file_off, file_off + cut).  Its size is known to within a few per cent
 // from the previous batch, so `read_threads` threads pread() disjoint pieces of that range at once and count
 // their line ends; nothing is carried over between batches (what lies behind the cut is read again next time,
 // from the page cache).
 int MateTextReader::next_plain(uint32_t max_reads, PinnedBuf& buf, uint64_t* bytes, uint32_t* n_reads) {
-    const uint64_t target = 4ull * max_reads;
+    const uint64_t target = rc.target(max_reads);
     *bytes = 0;
     *n_reads = 0;
     if (file_off >= file_size) {
@@ -467,7 +539,7 @@ int MateTextReader::next_plain(uint32_t max_reads, PinnedBuf& buf, uint64_t* byt
                 done += (size_t)got;
             }
             pc.got = (long)done;
-            pc.lines = count_newlines(buf.p + pc.begin, done);
+            pc.lines = rc.count(buf.p + pc.begin, done, 0);  // + the record start at its edge, below
         };
         std::vector<std::thread> helpers;
         for (int t = 1; t < nt; t++) helpers.emplace_back(work, t);
@@ -480,11 +552,13 @@ int MateTextReader::next_plain(uint32_t max_reads, PinnedBuf& buf, uint64_t* byt
             if ((size_t)pc.got != pc.len) short_read = true;
         }
         if (short_read) return io_fail(CSQ_ERR_IO, "%s: file changed while it was read", src.name.c_str());
-        // is the last line end of the batch inside this round?
+        // is the last line end (FASTA: the first record start behind the batch) inside this round?
         for (int t = 0; t < nt; t++) {
-            const Piece& pc = pieces[(size_t)t];
+            Piece& pc = pieces[(size_t)t];
+            const uint8_t prev = pc.begin ? buf.p[pc.begin - 1] : (uint8_t)'\n';
+            pc.lines += rc.edge(buf.p + pc.begin, pc.len, prev);
             if (lines + pc.lines >= target) {
-                const uint64_t rel = after_kth_newline(buf.p + pc.begin, pc.len, target - lines);
+                const uint64_t rel = rc.cut(buf.p + pc.begin, pc.len, target - lines, prev);
                 const size_t cut = pc.begin + (size_t)rel;
                 file_off += cut;
                 hint_bytes = cut;
@@ -508,7 +582,7 @@ int MateTextReader::next_plain(uint32_t max_reads, PinnedBuf& buf, uint64_t* byt
 int MateTextReader::next(uint32_t max_reads, PinnedBuf& buf, uint64_t* bytes, uint32_t* n_reads) {
     if (plain_file) return next_plain(max_reads, buf, bytes, n_reads);
     if (bgzf) return next_bgzf(max_reads, buf, bytes, n_reads);
-    const uint64_t target = 4ull * max_reads;
+    const uint64_t target = rc.target(max_reads);
     size_t piece = (size_t)max_reads * 512;
     piece = piece < (64u << 10) ? (64u << 10) : piece > (4u << 20) ? (4u << 20) : piece;
     size_t pos = 0;
@@ -524,9 +598,9 @@ int MateTextReader::next(uint32_t max_reads, PinnedBuf& buf, uint64_t* bytes, ui
         return io_fail(CSQ_ERR_NOMEM, "out of host memory for a batch of %u reads", max_reads);
     if (avail) {
         const uint8_t* c = carry.data() + carry_pos;
-        const uint64_t k = count_newlines(c, avail);
+        const uint64_t k = rc.count(c, avail, '\n');
         if (k >= target) {  // the batch is already here
-            const uint64_t cut = after_kth_newline(c, avail, target);
+            const uint64_t cut = rc.cut(c, avail, target, '\n');
             if (!buf.reserve((size_t)cut + 64, 0)) return io_fail(CSQ_ERR_NOMEM, "out of host memory for a batch of %u reads", max_reads);
             memcpy(buf.p, c, (size_t)cut);
             carry_pos += (size_t)cut;
@@ -554,11 +628,11 @@ int MateTextReader::next(uint32_t max_reads, PinnedBuf& buf, uint64_t* bytes, ui
         }
         last_start = pos;
         lines_before = lines;
-        lines += count_newlines(buf.p + pos, (size_t)got);
+        lines += rc.count(buf.p + pos, (size_t)got, pos ? buf.p[pos - 1] : (uint8_t)'\n');
         pos += (size_t)got;
     }
     if (lines >= target) {
-        const uint64_t rel = after_kth_newline(buf.p + last_start, pos - last_start, target - lines_before);
+        const uint64_t rel = rc.cut(buf.p + last_start, pos - last_start, target - lines_before, last_start ? buf.p[last_start - 1] : (uint8_t)'\n');
         const size_t cut = last_start + (size_t)rel;
         carry.assign(buf.p + cut, buf.p + pos);
         hint_bytes = cut;
@@ -626,12 +700,17 @@ int csq_text_reader_next_into(csq_text_reader* r, csqio::PinnedBuf* bufs /*[2]*/
 extern "C" {
 
 int csq_text_reader_open(const char* path1, const char* path2, csq_text_reader** out) {
+    return csq_text_reader_open_flags(path1, path2, 0, out);
+}
+
+int csq_text_reader_open_flags(const char* path1, const char* path2, uint32_t plan_flags, csq_text_reader** out) {
     if (!path1 || !out) {
         csq_set_error("null argument");
         return CSQ_ERR_INVALID;
     }
     csq_text_reader* r = new csq_text_reader();
     r->n_mates = path2 ? 2 : 1;
+    for (int m = 0; m < 2; m++) r->mate[m].rc.fasta = (plan_flags & CSQ_PLAN_FASTA) != 0;
     g_streams_side_by_side = r->n_mates;
     int rc = r->mate[0].open(path1);
     if (!rc && path2) rc = r->mate[1].open(path2);
@@ -689,6 +768,10 @@ uint64_t csq_count_newlines(const uint8_t* text, uint64_t n_bytes) { return text
 
 uint64_t csq_after_kth_newline(const uint8_t* text, uint64_t n_bytes, uint64_t k) {
     return text ? after_kth_newline(text, (size_t)n_bytes, k) : UINT64_MAX;
+}
+
+uint64_t csq_after_kth_fasta_record(const uint8_t* text, uint64_t n_bytes, uint64_t k) {
+    return text ? kth_fasta_record(text, (size_t)n_bytes, k + 1, '\n') : UINT64_MAX;
 }
 
 int csq_format_fastq(const csq_mate_in* mate, uint32_t n_reads, uint8_t* out, uint64_t capacity, uint64_t* bytes) {

@@ -70,6 +70,7 @@ def lib():
         L.csq_parse_fastq_mem.argtypes = [vp, C.c_uint64, u32, vp, vp, C.c_uint64, vp, vp, vp, C.c_uint64, vp,
                                           C.POINTER(u32), u64p, u64p]
         L.csq_text_reader_open.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(vp)]
+        L.csq_text_reader_open_flags.argtypes = [C.c_char_p, C.c_char_p, u32, C.POINTER(vp)]
         L.csq_text_reader_next.argtypes = [vp, i32, u32, C.POINTER(A.csq_batch_text)]
         L.csq_text_reader_close.argtypes = [vp]
         L.csq_text_reader_close.restype = None
@@ -77,6 +78,8 @@ def lib():
         L.csq_count_newlines.restype = C.c_uint64
         L.csq_after_kth_newline.argtypes = [vp, C.c_uint64, C.c_uint64]
         L.csq_after_kth_newline.restype = C.c_uint64
+        L.csq_after_kth_fasta_record.argtypes = [vp, C.c_uint64, C.c_uint64]
+        L.csq_after_kth_fasta_record.restype = C.c_uint64
         L.csq_gunzip_mem.argtypes = [vp, C.c_uint64, vp, C.c_uint64, C.c_uint64, u64p]
         L.csq_format_fastq.argtypes = [C.POINTER(A.csq_mate_in), u32, vp, C.c_uint64, u64p]
         L.csq_gz_deflate_host.argtypes = [vp, C.c_uint64, vp, C.c_uint64, u64p]
@@ -316,11 +319,13 @@ class BgzfRun:
 
 
 class TextReader:
-    """csq_text_reader: batches of raw FASTQ text cut at record boundaries (host side of the file driver)."""
+    """csq_text_reader: batches of raw FASTQ text cut at record boundaries (host side of the file driver).
+    flags = PLAN_FASTA: FASTA files, batches of whole FASTA records."""
 
-    def __init__(self, path1, path2=None):
+    def __init__(self, path1, path2=None, flags: int = 0):
         self._h = C.c_void_p()
-        check(lib().csq_text_reader_open(os.fsencode(path1), os.fsencode(path2) if path2 else None, C.byref(self._h)))
+        check(lib().csq_text_reader_open_flags(os.fsencode(path1), os.fsencode(path2) if path2 else None, flags,
+                                               C.byref(self._h)))
 
     def next(self, max_reads: int, buffer: int = 0):
         """-> (n_reads, [bytes per mate], first_record); n_reads == 0 at the end of the input."""

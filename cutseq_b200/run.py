@@ -218,13 +218,16 @@ def json_report(file, counters, prog, barcode, input1, input2, output1, output2,
 
 
 def _run_program(prog, inputs, outputs, settings):
+    from . import _abi as A
     from . import native
     from .transcode import Transcoders
 
-    # .bz2 / .xz files (xopen handles them in the reference) go through named pipes and Python's codecs
-    with Transcoders(inputs, outputs) as tc:
+    # .bz2 / .xz files (xopen handles them in the reference) go through named pipes and Python's codecs; FASTA files
+    # are parsed and written by the library itself (CSQ_PLAN_FASTA)
+    with Transcoders(inputs, outputs, fasta_native=True) as tc:
         return native.run_files(prog, tc.inputs, tc.outputs, gpus=getattr(settings, "gpus", 1),
-                                threads=settings.threads, batch_reads=getattr(settings, "batch_reads", 0))
+                                threads=settings.threads, batch_reads=getattr(settings, "batch_reads", 0),
+                                flags=A.PLAN_FASTA if tc.fasta_native else 0)
 
 
 def pipeline_single(input1, output1, short1, untrimmed1, barcode, settings):

@@ -9,9 +9,11 @@ work): the library sees a plain FASTQ stream, nothing below the C ABI changes.  
 and such files are refused with a clear message instead of being misread as plain text.
 
 FASTA input (records without qualities; the reference hands ``qualities=has_qualities()`` on to its output files,
-run.py:439, 756) takes the same route: the pump turns every record into a FASTQ record with a constant quality far above
-any cutoff - quality trimming has nothing to remove, as for a read without qualities - and the output pumps write
-``>name`` / sequence records again (dnaio's FASTA writer does not wrap lines), compressed as the file name says.
+run.py:439, 756) is read and written by the library itself (``CSQ_PLAN_FASTA``; ``Transcoders(..., fasta_native=True)``
+leaves such files alone but for their compression).  The converting pumps below stay as the reference the library is
+tested against: the pump turns every record into a FASTQ record with a constant quality far above any cutoff - quality
+trimming has nothing to remove, as for a read without qualities - and the output pumps write ``>name`` / sequence
+records again (dnaio's FASTA writer does not wrap lines), compressed as the file name says.
 (Whether the reference itself survives FASTA input is doubtful - run.py:416 / 720 always add cutadapt's QualityTrimmer,
 which takes the length of ``read.qualities`` - see DESIGN.md section 7; here such input simply works.)
 """
@@ -173,9 +175,13 @@ def fastq_to_fasta(src, dst):
 
 
 class Transcoders:
-    """Context manager: ``tc.inputs`` / ``tc.outputs`` are what the library should open instead of the given paths."""
+    """Context manager: ``tc.inputs`` / ``tc.outputs`` are what the library should open instead of the given paths.
 
-    def __init__(self, inputs, outputs):
+    ``tc.fasta`` tells whether the inputs are FASTA, ``tc.fasta_native`` whether the library is to read them as such.  By default FASTA goes through the converting pumps (the library
+    sees FASTQ); with ``fasta_native=True`` only compressions the library cannot read or write get a pump, and the
+    caller runs the library with ``CSQ_PLAN_FASTA``."""
+
+    def __init__(self, inputs, outputs, fasta_native=False):
         self.inputs = list(inputs)
         self.outputs = {k: list(v) if v else v for k, v in outputs.items()}
         self._threads = []  # (thread, fifo, "in" | "out")
@@ -187,7 +193,9 @@ class Transcoders:
         self.fasta = bool(fasta) and all(fasta)
         if any(fasta) and not self.fasta:
             raise ValueError("the input files differ in format (FASTA and FASTQ)")
-        if self.fasta:  # every input and every output goes through a converting pump
+        self.fasta_native = self.fasta and fasta_native  # the library reads and writes these FASTA files itself
+        self._convert = self.fasta and not fasta_native
+        if self._convert:  # every input and every output goes through a converting pump
             self._in_jobs = [(i, p, _reader(p)) for i, p, _ in in_jobs if p]
             self._out_jobs = [(k, m, p, _writer(p)) for k, m, p, _ in out_jobs if p]
         else:
@@ -202,12 +210,12 @@ class Transcoders:
             fifo = os.path.join(self._tmp, f"in_{i}.fq")
             os.mkfifo(fifo)
             self.inputs[i] = fifo
-            self._start(self._feed_fasta if self.fasta else self._feed, (path, opener, fifo), fifo, "in")
+            self._start(self._feed_fasta if self._convert else self._feed, (path, opener, fifo), fifo, "in")
         for k, m, path, opener in self._out_jobs:
             fifo = os.path.join(self._tmp, f"out_{k}_{m}.fq")  # no compression suffix: the library writes plain text
             os.mkfifo(fifo)
             self.outputs[k][m] = fifo
-            self._start(self._drain_fasta if self.fasta else self._drain, (path, opener, fifo), fifo, "out")
+            self._start(self._drain_fasta if self._convert else self._drain, (path, opener, fifo), fifo, "out")
         return self
 
     def _start(self, fn, args, fifo, side):

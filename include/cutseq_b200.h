@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define CSQ_ABI_VERSION 2
+#define CSQ_ABI_VERSION 3
 
 typedef enum csq_status {
     CSQ_OK = 0,
@@ -164,6 +164,12 @@ typedef struct csq_text_in {
     uint64_t bytes;
 } csq_text_in;
 
+/* Under CSQ_PLAN_FASTA a text batch holds FASTA records instead: a record starts at a line whose first byte is '>'; the
+ * header is the rest of that line without its trailing '\r' / '\n' bytes; the sequence is the concatenation of the
+ * following lines up to the next header, each stripped of leading and trailing ASCII whitespace (blank lines and empty
+ * sequences are allowed).  Blank lines may stand in front of the first header; any other text there is CSQ_ERR_FORMAT.
+ * n_reads is the number of headers; a batch holding a different number is CSQ_ERR_FORMAT.  The last line must be
+ * ended by '\n' as for FASTQ.  A FASTA read is trimmed as if every quality were 'I' (Q40 at base 33). */
 typedef struct csq_batch_text {
     uint32_t n_reads;          /* records per mate in this batch                       */
     uint32_t n_mates;          /* 1 or 2                                               */
@@ -255,6 +261,9 @@ typedef struct csq_plan csq_plan;
                                      csq_text_out.bytes = compressed bytes; what xopen does behind the reference's
                                      default .fastq.gz outputs (run.py:1058-1093), without the text crossing PCIe    */
 #define CSQ_PLAN_NO_EXACT_STOP 1024u /* exact DP walks every column even after an error-free full match (results are the same; A/B) */
+#define CSQ_PLAN_FASTA 8192u     /* text batches (csq_submit_text, csq_upload_text) hold FASTA records and the emitters write FASTA
+                                     (">name\nsequence\n", not wrapped); see csq_batch_text.  csq_submit, csq_upload,
+                                     csq_submit_bgzf and csq_bgzf_count_lines return CSQ_ERR_INVALID under this flag          */
 /* (flag values 8, 16, 32, 128, 512, 2048 selected slower kernel variants in round 1 - per-pair / 8- / 32-lane emitters,
  * one-pass parse, one-lane / one-column homopolymer DP; those kernels were removed after measurement and the bits are ignored) */
 
@@ -350,12 +359,19 @@ int csq_parse_fastq_mem(const uint8_t* text, uint64_t n_bytes, uint32_t max_read
  * on the host: the stream is cut after 4 * max_reads line ends. in->n_reads == 0 at the end. */
 typedef struct csq_text_reader csq_text_reader;
 int csq_text_reader_open(const char* path1, const char* path2, csq_text_reader** out);
+/* The same with plan flags: under CSQ_PLAN_FASTA the files are FASTA and the stream is cut in front of the
+ * (max_reads + 1)-th record start instead (batches hold max_reads records; see csq_batch_text).  BGZF-framed files are
+ * read like any gzip file. */
+int csq_text_reader_open_flags(const char* path1, const char* path2, uint32_t plan_flags, csq_text_reader** out);
 int csq_text_reader_next(csq_text_reader* r, int buffer, uint32_t max_reads, csq_batch_text* in);
 void csq_text_reader_close(csq_text_reader* r);
 /* Text-batch helpers (host, SIMD): number of '\n' in [text, text + n_bytes); and the offset
  * one past the k-th '\n' (k >= 1), or UINT64_MAX when there are fewer. */
 uint64_t csq_count_newlines(const uint8_t* text, uint64_t n_bytes);
 uint64_t csq_after_kth_newline(const uint8_t* text, uint64_t n_bytes, uint64_t k);
+/* FASTA twin (host, SIMD): the offset of the (k+1)-th record start ('>' as the first byte of a line; the text starts at
+ * a line start) in [text, text + n_bytes), or UINT64_MAX when there are fewer.  k = 0: the first record start. */
+uint64_t csq_after_kth_fasta_record(const uint8_t* text, uint64_t n_bytes, uint64_t k);
 /* gzip data in memory -> dst, decoded in pieces of `piece` bytes with the library's own inflate (tests). */
 int csq_gunzip_mem(const uint8_t* src, uint64_t n, uint8_t* dst, uint64_t cap, uint64_t piece, uint64_t* out_n);
 /* The device gzip writer's algorithm run on the host, piece by piece (CPU tests of the code construction, the block
@@ -372,7 +388,8 @@ int csq_format_fastq(const csq_mate_in* mate, uint32_t n_reads, uint8_t* out, ui
                      uint64_t* bytes);
 
 /* Whole-file driver: read -> (double-buffered) GPU chain -> ordered write. Output paths
- * may be NULL (destination discarded); a ".gz" suffix selects gzip output. */
+ * may be NULL (destination discarded); a ".gz" suffix selects gzip output.  With CSQ_PLAN_FASTA in plan_flags the
+ * inputs are FASTA files (plain or gzip) and the outputs FASTA. */
 typedef struct csq_files {
     const char* in[2];
     const char* out[CSQ_N_DEST][2];
