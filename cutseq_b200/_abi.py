@@ -4,7 +4,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 CSQ_MAX_ADAPTER = 128
 CSQ_MAX_READ_LEN = 895

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcutseq_b200.so")
-SOURCES = ["kernels.cu", "tail.cu", "emit_stage.cu", "gz_deflate.cu", "gz_inflate.cu", "plan.cu", "prefilter.cu", "parse.cu", "synth.cu", "fastq_io.cpp", "text_reader.cpp", "inflate.cpp", "pinflate.cpp", "pipeline.cpp", "host_numa.cpp"]
+SOURCES = ["kernels.cu", "tail.cu", "emit_stage.cu", "gz_deflate.cu", "gz_inflate.cu", "gz_stream.cu", "plan.cu", "prefilter.cu", "parse.cu", "synth.cu", "fastq_io.cpp", "text_reader.cpp", "inflate.cpp", "pinflate.cpp", "pipeline.cpp", "host_numa.cpp"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC,-O3,-pthread,-Wall", "-cudart", "static",

@@ -36,6 +36,12 @@
 #define GZI_FFS(x) __builtin_ffs((int)(x))
 #endif
 
+#if defined(__GNUC__) && !defined(__CUDA_ARCH__)
+// the match copies store v[k] only under the condition they loaded it under
+#pragma GCC diagnostic push
+#pragma GCC diagnostic ignored "-Wmaybe-uninitialized"
+#endif
+
 namespace gzi {
 
 // The cooperating lanes: a whole warp or an aligned part of one (LANES = 16: two members per warp, each instruction
@@ -60,7 +66,8 @@ struct Group {
 constexpr int MAXBITS = 15, MAXLCODES = 286, MAXDCODES = 30, FIXLCODES = 288;
 constexpr int LBITS = 10, DBITS = 8;  // index bits of the direct tables
 
-enum Status { OK = 0, ERR_HEADER = 1, ERR_BLOCK = 2, ERR_CODE = 3, ERR_DIST = 4, ERR_OVERRUN = 5, ERR_TRAILER = 6 };
+// (8 and up: 7 is k_gz_check's CRC-32 mismatch)
+enum Status { OK = 0, ERR_HEADER = 1, ERR_BLOCK = 2, ERR_CODE = 3, ERR_DIST = 4, ERR_OVERRUN = 5, ERR_TRAILER = 6, ERR_INPUT = 8 };
 
 struct Tables {  // per group (device: shared memory, 6.1 KB per group)
     // entries: code length [3:0] | extra bits [7:4] | base value [23:8] | LIT bit 31 | EOB bit 30; 0: the code is longer
@@ -273,15 +280,15 @@ GZI_HD int construct(uint16_t* count, uint16_t* symbol, uint32_t* lut, const uin
 // `len` bytes at d are the bytes `dist` in front of them, by all lanes: byte i of the match is byte (i mod dist) of the
 // `dist` bytes in front of it, which all exist already - no lane waits for another one's store.  The loads of a long
 // copy are issued before its first store.
-template <int LANES>
-GZI_HD void copy_match(uint8_t* d, uint32_t dist, uint32_t len, int lane) {  // (no synchronisation inside)
-    const uint8_t* sp = d - dist;
+template <int LANES, typename Sym>
+GZI_HD void copy_match(Sym* d, uint32_t dist, uint32_t len, int lane) {  // (no synchronisation inside)
+    const Sym* sp = d - dist;
     if (dist >= len) {
         if (len <= (uint32_t)LANES) {
             if ((uint32_t)lane < len) d[lane] = sp[lane];
         } else {
             for (uint32_t base = 0; base < len; base += 4u * LANES) {
-                uint8_t v[4];
+                Sym v[4];
                 GZI_UNROLL
                 for (uint32_t k = 0; k < 4; k++) {
                     const uint32_t i = base + k * LANES + (uint32_t)lane;
@@ -295,7 +302,7 @@ GZI_HD void copy_match(uint8_t* d, uint32_t dist, uint32_t len, int lane) {  // 
             }
         }
     } else if (dist == 1) {  // a run of one byte
-        const uint8_t c = sp[0];
+        const Sym c = sp[0];
         for (uint32_t i = (uint32_t)lane; i < len; i += LANES) d[i] = c;
     } else {  // a period shorter than the match
         uint32_t r = (uint32_t)lane % dist;
@@ -308,11 +315,232 @@ GZI_HD void copy_match(uint8_t* d, uint32_t dist, uint32_t len, int lane) {  // 
     }
 }
 
+// Dynamic block header at the reader's position (behind the 3 header bits) -> both codes in T.  The code-length code
+// must be complete, the literal/length code must have an end-of-block code, and an incomplete code is only accepted for
+// a single code of one bit.
+template <int LANES>
+GZI_HD int read_dynamic(BitIn& b, Tables& T, const Group<LANES>& G) {
+    const int lane = G.lane;
+    refill(b);
+    const int nlen = (int)take(b, 5) + 257, ndist = (int)take(b, 5) + 1, ncode = (int)take(b, 4) + 4;
+    if (nlen > MAXLCODES || ndist > MAXDCODES) return ERR_CODE;
+    // the code-length code: 19 lengths of 3 bits in a fixed order, read by every lane, stored by lane 0
+    uint32_t packed[2] = {0, 0};  // 19 x 3 bits, by position in the stream
+    for (int idx = 0; idx < ncode; idx++) {
+        refill(b);
+        const uint32_t v = take(b, 3);
+        if (idx < 10)
+            packed[0] |= v << (3 * idx);
+        else
+            packed[1] |= v << (3 * (idx - 10));
+    }
+    G.sync();
+    if (lane == 0) {
+        const uint8_t order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
+        for (int idx = 0; idx < 19; idx++) {
+            const uint32_t v = idx < 10 ? (packed[0] >> (3 * idx)) & 7u : (packed[1] >> (3 * (idx - 10))) & 7u;
+            T.lengths[order[idx]] = (uint8_t)(idx < ncode ? v : 0u);
+        }
+    }
+    G.sync();
+    // its tables live where the distance tables will be (19 symbols, codes of at most 7 bits <= DBITS)
+    if (construct<LANES, DBITS, 0>(T.dcount, T.dsym, T.dlut, T.lengths, 19, G) != 0) return ERR_CODE;  // must be complete
+    int idx = 0, prev = 0;
+    bool have_eob = false;
+    while (idx < nlen + ndist) {
+        refill(b);
+        const uint32_t ce = decode_entry<DBITS, 0>(b, T.dlut, T.dcount, T.dsym);
+        if (ce == 0xFFFFFFFFu) return ERR_CODE;
+        const int sym = (int)(ce >> 8);
+        int rep = 1, val = sym;
+        if (sym == 16) {
+            if (idx == 0) return ERR_CODE;
+            val = prev;
+            rep = 3 + (int)take(b, 2);
+        } else if (sym == 17) {
+            val = 0;
+            rep = 3 + (int)take(b, 3);
+        } else if (sym == 18) {
+            val = 0;
+            rep = 11 + (int)take(b, 7);
+        }
+        if (idx + rep > nlen + ndist) return ERR_CODE;
+        if (val != 0 && idx <= 256 && idx + rep > 256) have_eob = true;
+        // literal/length lengths at [0, nlen), distance lengths behind them at [nlen, nlen + ndist)
+        for (int r = lane; r < rep; r += LANES) T.lengths[idx + r] = (uint8_t)val;
+        idx += rep;
+        prev = val;
+    }
+    if (!have_eob) return ERR_CODE;  // no end-of-block code
+    G.sync();
+    // the distance code first: the code-length tables in its place are done with
+    int err = construct<LANES, DBITS, 2>(T.dcount, T.dsym, T.dlut, T.lengths + nlen, ndist, G);
+    if (err < 0 || (err > 0 && ndist - (int)T.dcount[0] != 1)) return ERR_CODE;
+    err = construct<LANES, LBITS, 1>(T.lcount, T.lsym, T.llut, T.lengths, nlen, G);
+    if (err < 0 || (err > 0 && nlen - (int)T.lcount[0] != 1)) return ERR_CODE;
+    return OK;
+}
+
+// One DEFLATE block at the reader's position -> dst[out ..), out advanced; *last = its BFINAL bit.  Sym is the output
+// type: bytes for a gzip member, 16-bit symbols for a span of a stream decoded without its window (gz_stream.cu: a
+// reference in front of the span copies the marker 0x8000 | place like any byte).  dst[0 .. out) is what a distance
+// may reach.  ERR_OVERRUN: the block does not fit in cap (nothing past cap is written); ERR_INPUT: it runs past b.end.
+template <int LANES, typename Sym>
+GZI_HD int inflate_block(BitIn& b, Sym* dst, uint32_t& out, uint32_t cap, Tables& T, const Group<LANES>& G, int* last) {
+    const int lane = G.lane;
+    refill(b);
+    *last = (int)take(b, 1);
+    const uint32_t type = take(b, 2);
+    if (type == 0) {  // stored
+        take(b, b.cnt & 7);  // to the byte boundary
+        refill(b);
+        const uint32_t len = take(b, 16);
+        refill(b);
+        const uint32_t nlen = take(b, 16);
+        if ((len ^ 0xFFFFu) != nlen) return ERR_BLOCK;
+        const uint8_t* q = byte_pos(b);  // the whole bytes in the bit buffer are given back
+        if (q + len > b.end) return ERR_INPUT;
+        if (out + len > cap) return ERR_OVERRUN;
+        for (uint32_t i = (uint32_t)lane; i < len; i += LANES) dst[out + i] = q[i];
+        out += len;
+        start(b, q + len);
+        return OK;
+    }
+    if (type == 3) return ERR_BLOCK;
+    if (type == 1) {  // fixed codes
+        G.sync();
+        for (int s = lane; s < FIXLCODES; s += LANES) T.lengths[s] = (uint8_t)(s < 144 ? 8 : s < 256 ? 9 : s < 280 ? 7 : 8);
+        for (int s = lane; s < MAXDCODES; s += LANES) T.lengths[FIXLCODES + s] = 5;
+        G.sync();
+        construct<LANES, LBITS, 1>(T.lcount, T.lsym, T.llut, T.lengths, FIXLCODES, G);
+        construct<LANES, DBITS, 2>(T.dcount, T.dsym, T.dlut, T.lengths + FIXLCODES, MAXDCODES, G);
+    } else {  // dynamic codes
+        const int rc = read_dynamic<LANES>(b, T, G);
+        if (rc != OK) return rc;
+    }
+    constexpr uint32_t CHUNK = 8;           // bytes a lane has in flight
+    constexpr uint32_t SHORT = 2 * CHUNK;   // longer matches are copied by all lanes
+    bool eob = false;
+    while (!eob) {  // batches of up to LANES tokens
+        // a batch reads at most LANES * 6 bytes: the input is padded behind b.end
+        if (b.p > b.end + 8) return ERR_INPUT;
+        uint32_t my_off = 0, my_tok = 0;  // token `lane`: distance << 16 | length, or (distance 0) the literal
+        uint32_t ntok = 0;
+        while (ntok < (uint32_t)LANES) {
+            refill(b);
+            uint32_t e = decode_entry<LBITS, 1>(b, T.llut, T.lcount, T.lsym);
+            uint32_t len = 1, tok;
+            if (e >= 0x01000000u) {  // a literal, the end of the block or an invalid code
+                if (e == 0xFFFFFFFFu) return ERR_CODE;
+                if (e & E_EOB) {
+                    eob = true;
+                    break;
+                }
+                tok = (e >> 8) & 0xFFu;
+            } else {  // a match: base length + extra bits, then the distance likewise
+                const uint32_t x = e >> 4 & 15u;
+                len = (e >> 8) + ((uint32_t)b.buf & ~(0xFFFFFFFFu << x));
+                b.buf >>= x;
+                b.cnt -= (int)x;
+                refill_rare(b);
+                e = decode_entry<DBITS, 2>(b, T.dlut, T.dcount, T.dsym);
+                if (e == 0xFFFFFFFFu) return ERR_DIST;
+                const uint32_t y = e >> 4 & 15u;
+                const uint32_t dist = (e >> 8) + ((uint32_t)b.buf & ~(0xFFFFFFFFu << y));
+                b.buf >>= y;
+                b.cnt -= (int)y;
+                if (dist > out) return ERR_DIST;
+                tok = (dist << 16) | len;
+            }
+            if ((uint32_t)lane == ntok) {
+                my_off = out;
+                my_tok = tok;
+            }
+            out += len;
+            ntok++;
+        }
+        if (out > cap) return ERR_OVERRUN;  // nothing of the batch has been written yet
+        const uint32_t my_dist = my_tok >> 16, my_len = my_dist ? (my_tok & 0xFFFFu) : 1u, my_lit = my_tok & 0xFFu;
+        // ---- resolve the batch ----
+        bool pending = (uint32_t)lane < ntok;
+        if (pending && my_dist == 0) {
+            dst[my_off] = (Sym)my_lit;
+            pending = false;
+        }
+        G.sync();  // literals, stored blocks and earlier batches are visible to every lane
+        for (;;) {
+            const uint32_t wait = G.ballot(pending);
+            if (!wait) break;
+            const int first = GZI_FFS(wait) - 1;
+            const uint32_t upto = G.shfl(my_off, first);  // every byte in front of the first unfinished token is written
+            const uint32_t flen = G.shfl(my_len, first);
+            if (flen > SHORT) {  // a long match: its source is complete, all lanes copy it
+                copy_match<LANES, Sym>(dst + upto, G.shfl(my_dist, first), flen, lane);
+                if (lane == first) pending = false;
+            } else {
+                // short matches whose source is complete (the first unfinished one always is), each by its own lane;
+                // byte i is byte (i mod dist) of the dist bytes in front of the match.  (Exact dependencies - the
+                // tokens of the batch that write the source instead of "everything in front of the first unfinished
+                // one" - need fewer rounds but 64 shuffles per batch and 26 more registers: measured, slower.)
+                const bool ready = pending && my_len <= SHORT && my_off - my_dist + (my_len < my_dist ? my_len : my_dist) <= upto;
+                const bool more = G.ballot(ready && my_len > CHUNK) != 0;
+                if (ready) {
+                    Sym* d = dst + my_off;
+                    const Sym* sp = d - my_dist;
+                    uint32_t r = 0;
+                    Sym v[CHUNK];
+                    GZI_UNROLL
+                    for (uint32_t k = 0; k < CHUNK; k++)
+                        if (k < my_len) {
+                            v[k] = sp[r];
+                            r = r + 1 == my_dist ? 0 : r + 1;
+                        }
+                    GZI_UNROLL
+                    for (uint32_t k = 0; k < CHUNK; k++)
+                        if (k < my_len) d[k] = v[k];
+                    if (more) {  // (uniform) the second half of the longer ones
+                        GZI_UNROLL
+                        for (uint32_t k = CHUNK; k < SHORT; k++)
+                            if (k < my_len) {
+                                v[k - CHUNK] = sp[r];
+                                r = r + 1 == my_dist ? 0 : r + 1;
+                            }
+                        GZI_UNROLL
+                        for (uint32_t k = CHUNK; k < SHORT; k++)
+                            if (k < my_len) d[k] = v[k - CHUNK];
+                    }
+                    pending = false;
+                }
+            }
+            G.sync();  // this round's stores are visible to the next one's loads
+        }
+    }
+    return OK;
+}
+
+// Byte offset of the first DEFLATE block of the gzip member whose header starts at src[0] (n bytes readable), 0 when
+// the header is not one (magic, CM = 8, reserved FLG bits clear) or does not end inside the n bytes.
+GZI_HD uint32_t gzip_header_size(const uint8_t* src, uint32_t n) {
+    if (n < 18 || src[0] != 0x1f || src[1] != 0x8b || src[2] != 8 || (src[3] & 0xE0u)) return 0;
+    const uint32_t flg = src[3];
+    uint32_t pos = 10;
+    if (flg & 4u) pos = 12 + (src[10] | ((uint32_t)src[11] << 8));
+    if (flg & 8u) {
+        while (pos < n && src[pos]) pos++;
+        pos++;
+    }
+    if (flg & 16u) {
+        while (pos < n && src[pos]) pos++;
+        pos++;
+    }
+    if (flg & 2u) pos += 2;
+    return pos < n ? pos : 0;
+}
+
 // One gzip member src[0 .. n) -> dst[0 .. cap).  *produced = bytes written (valid in every lane).  Checks ISIZE and
 // that the member ends where it should; the CRC-32 of the text is verified by the caller (k_gz_check / the host twin).
 template <int LANES>
 GZI_HD int inflate_member(const uint8_t* src, uint32_t n, uint8_t* dst, uint32_t cap, Tables& T, const Group<LANES>& G, uint32_t* produced) {
-    const int lane = G.lane;
     *produced = 0;
     // gzip header (RFC 1952): magic, CM = 8, FLG, MTIME(4), XFL, OS, then the optional fields
     if (n < 18 || src[0] != 0x1f || src[1] != 0x8b || src[2] != 8) return ERR_HEADER;
@@ -338,185 +566,8 @@ GZI_HD int inflate_member(const uint8_t* src, uint32_t n, uint8_t* dst, uint32_t
     uint32_t out = 0;  // bytes produced
     int last;
     do {
-        refill(b);
-        last = (int)take(b, 1);
-        const uint32_t type = take(b, 2);
-        if (type == 0) {  // stored
-            take(b, b.cnt & 7);  // to the byte boundary
-            refill(b);
-            const uint32_t len = take(b, 16);
-            refill(b);
-            const uint32_t nlen = take(b, 16);
-            if ((len ^ 0xFFFFu) != nlen) return ERR_BLOCK;
-            const uint8_t* q = byte_pos(b);  // the whole bytes in the bit buffer are given back
-            if (q + len > b.end || out + len > cap) return ERR_OVERRUN;
-            for (uint32_t i = (uint32_t)lane; i < len; i += LANES) dst[out + i] = q[i];
-            out += len;
-            start(b, q + len);
-            continue;
-        }
-        if (type == 3) return ERR_BLOCK;
-        if (type == 1) {  // fixed codes
-            G.sync();
-            for (int s = lane; s < FIXLCODES; s += LANES) T.lengths[s] = (uint8_t)(s < 144 ? 8 : s < 256 ? 9 : s < 280 ? 7 : 8);
-            for (int s = lane; s < MAXDCODES; s += LANES) T.lengths[FIXLCODES + s] = 5;
-            G.sync();
-            construct<LANES, LBITS, 1>(T.lcount, T.lsym, T.llut, T.lengths, FIXLCODES, G);
-            construct<LANES, DBITS, 2>(T.dcount, T.dsym, T.dlut, T.lengths + FIXLCODES, MAXDCODES, G);
-        } else {  // dynamic codes
-            refill(b);
-            const int nlen = (int)take(b, 5) + 257, ndist = (int)take(b, 5) + 1, ncode = (int)take(b, 4) + 4;
-            if (nlen > MAXLCODES || ndist > MAXDCODES) return ERR_CODE;
-            // the code-length code: 19 lengths of 3 bits in a fixed order, read by every lane, stored by lane 0
-            uint32_t packed[2] = {0, 0};  // 19 x 3 bits, by position in the stream
-            for (int idx = 0; idx < ncode; idx++) {
-                refill(b);
-                const uint32_t v = take(b, 3);
-                if (idx < 10)
-                    packed[0] |= v << (3 * idx);
-                else
-                    packed[1] |= v << (3 * (idx - 10));
-            }
-            G.sync();
-            if (lane == 0) {
-                const uint8_t order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
-                for (int idx = 0; idx < 19; idx++) {
-                    const uint32_t v = idx < 10 ? (packed[0] >> (3 * idx)) & 7u : (packed[1] >> (3 * (idx - 10))) & 7u;
-                    T.lengths[order[idx]] = (uint8_t)(idx < ncode ? v : 0u);
-                }
-            }
-            G.sync();
-            // its tables live where the distance tables will be (19 symbols, codes of at most 7 bits <= DBITS)
-            if (construct<LANES, DBITS, 0>(T.dcount, T.dsym, T.dlut, T.lengths, 19, G) != 0) return ERR_CODE;  // must be complete
-            int idx = 0, prev = 0;
-            bool have_eob = false;
-            while (idx < nlen + ndist) {
-                refill(b);
-                const uint32_t ce = decode_entry<DBITS, 0>(b, T.dlut, T.dcount, T.dsym);
-                if (ce == 0xFFFFFFFFu) return ERR_CODE;
-                const int sym = (int)(ce >> 8);
-                int rep = 1, val = sym;
-                if (sym == 16) {
-                    if (idx == 0) return ERR_CODE;
-                    val = prev;
-                    rep = 3 + (int)take(b, 2);
-                } else if (sym == 17) {
-                    val = 0;
-                    rep = 3 + (int)take(b, 3);
-                } else if (sym == 18) {
-                    val = 0;
-                    rep = 11 + (int)take(b, 7);
-                }
-                if (idx + rep > nlen + ndist) return ERR_CODE;
-                if (val != 0 && idx <= 256 && idx + rep > 256) have_eob = true;
-                // literal/length lengths at [0, nlen), distance lengths behind them at [nlen, nlen + ndist)
-                for (int r = lane; r < rep; r += LANES) T.lengths[idx + r] = (uint8_t)val;
-                idx += rep;
-                prev = val;
-            }
-            if (!have_eob) return ERR_CODE;  // no end-of-block code
-            G.sync();
-            // the distance code first: the code-length tables in its place are done with
-            int err = construct<LANES, DBITS, 2>(T.dcount, T.dsym, T.dlut, T.lengths + nlen, ndist, G);
-            if (err < 0 || (err > 0 && ndist - (int)T.dcount[0] != 1)) return ERR_CODE;
-            err = construct<LANES, LBITS, 1>(T.lcount, T.lsym, T.llut, T.lengths, nlen, G);
-            if (err < 0 || (err > 0 && nlen - (int)T.lcount[0] != 1)) return ERR_CODE;
-        }
-        constexpr uint32_t CHUNK = 8;           // bytes a lane has in flight
-        constexpr uint32_t SHORT = 2 * CHUNK;   // longer matches are copied by all lanes
-        bool eob = false;
-        while (!eob) {  // batches of up to LANES tokens
-            uint32_t my_off = 0, my_tok = 0;  // token `lane`: distance << 16 | length, or (distance 0) the literal
-            uint32_t ntok = 0;
-            while (ntok < (uint32_t)LANES) {
-                refill(b);
-                uint32_t e = decode_entry<LBITS, 1>(b, T.llut, T.lcount, T.lsym);
-                uint32_t len = 1, tok;
-                if (e >= 0x01000000u) {  // a literal, the end of the block or an invalid code
-                    if (e == 0xFFFFFFFFu) return ERR_CODE;
-                    if (e & E_EOB) {
-                        eob = true;
-                        break;
-                    }
-                    tok = (e >> 8) & 0xFFu;
-                } else {  // a match: base length + extra bits, then the distance likewise
-                    const uint32_t x = e >> 4 & 15u;
-                    len = (e >> 8) + ((uint32_t)b.buf & ~(0xFFFFFFFFu << x));
-                    b.buf >>= x;
-                    b.cnt -= (int)x;
-                    refill_rare(b);
-                    e = decode_entry<DBITS, 2>(b, T.dlut, T.dcount, T.dsym);
-                    if (e == 0xFFFFFFFFu) return ERR_DIST;
-                    const uint32_t y = e >> 4 & 15u;
-                    const uint32_t dist = (e >> 8) + ((uint32_t)b.buf & ~(0xFFFFFFFFu << y));
-                    b.buf >>= y;
-                    b.cnt -= (int)y;
-                    if (dist > out) return ERR_DIST;
-                    tok = (dist << 16) | len;
-                }
-                if ((uint32_t)lane == ntok) {
-                    my_off = out;
-                    my_tok = tok;
-                }
-                out += len;
-                ntok++;
-            }
-            if (out > cap) return ERR_OVERRUN;  // nothing of the batch has been written yet
-            const uint32_t my_dist = my_tok >> 16, my_len = my_dist ? (my_tok & 0xFFFFu) : 1u, my_lit = my_tok & 0xFFu;
-            // ---- resolve the batch ----
-            bool pending = (uint32_t)lane < ntok;
-            if (pending && my_dist == 0) {
-                dst[my_off] = (uint8_t)my_lit;
-                pending = false;
-            }
-            G.sync();  // literals, stored blocks and earlier batches are visible to every lane
-            for (;;) {
-                const uint32_t wait = G.ballot(pending);
-                if (!wait) break;
-                const int first = GZI_FFS(wait) - 1;
-                const uint32_t upto = G.shfl(my_off, first);  // every byte in front of the first unfinished token is written
-                const uint32_t flen = G.shfl(my_len, first);
-                if (flen > SHORT) {  // a long match: its source is complete, all lanes copy it
-                    copy_match<LANES>(dst + upto, G.shfl(my_dist, first), flen, lane);
-                    if (lane == first) pending = false;
-                } else {
-                    // short matches whose source is complete (the first unfinished one always is), each by its own lane;
-                    // byte i is byte (i mod dist) of the dist bytes in front of the match.  (Exact dependencies - the
-                    // tokens of the batch that write the source instead of "everything in front of the first unfinished
-                    // one" - need fewer rounds but 64 shuffles per batch and 26 more registers: measured, slower.)
-                    const bool ready = pending && my_len <= SHORT && my_off - my_dist + (my_len < my_dist ? my_len : my_dist) <= upto;
-                    const bool more = G.ballot(ready && my_len > CHUNK) != 0;
-                    if (ready) {
-                        uint8_t* d = dst + my_off;
-                        const uint8_t* sp = d - my_dist;
-                        uint32_t r = 0;
-                        uint8_t v[CHUNK];
-                        GZI_UNROLL
-                        for (uint32_t k = 0; k < CHUNK; k++)
-                            if (k < my_len) {
-                                v[k] = sp[r];
-                                r = r + 1 == my_dist ? 0 : r + 1;
-                            }
-                        GZI_UNROLL
-                        for (uint32_t k = 0; k < CHUNK; k++)
-                            if (k < my_len) d[k] = v[k];
-                        if (more) {  // (uniform) the second half of the longer ones
-                            GZI_UNROLL
-                            for (uint32_t k = CHUNK; k < SHORT; k++)
-                                if (k < my_len) {
-                                    v[k - CHUNK] = sp[r];
-                                    r = r + 1 == my_dist ? 0 : r + 1;
-                                }
-                            GZI_UNROLL
-                            for (uint32_t k = CHUNK; k < SHORT; k++)
-                                if (k < my_len) d[k] = v[k - CHUNK];
-                        }
-                        pending = false;
-                    }
-                }
-                G.sync();  // this round's stores are visible to the next one's loads
-            }
-        }
+        const int rc = inflate_block<LANES, uint8_t>(b, dst, out, cap, T, G, &last);
+        if (rc != OK) return rc;
     } while (!last);
     G.sync();
     // trailer: CRC-32 (verified by the caller), ISIZE
@@ -529,3 +580,7 @@ GZI_HD int inflate_member(const uint8_t* src, uint32_t n, uint8_t* dst, uint32_t
 }
 
 }  // namespace gzi
+
+#if defined(__GNUC__) && !defined(__CUDA_ARCH__)
+#pragma GCC diagnostic pop
+#endif

@@ -133,6 +133,30 @@ class ParallelInflater {
     Impl* p_;
 };
 
+// Ordinary gzip files decoded on a GPU (gz_stream.cu, csq_gz_stream_inflate), or by its host twin (device < 0): same
+// interface as Inflater.  (The file driver keeps ParallelInflater: on one B200 box this decoder was measured slower on
+// the files.gzip workload, DESIGN.md section 4.6.)
+// Span and round sizes in compressed bytes, 0: the default (CSQ_GZ_STREAM_SPAN / CSQ_GZ_STREAM_ROUND, else 128 KiB and
+// 64 MiB).  chain_log, when given, receives every span of the decode chain in file order.
+struct ChainEntry {
+    uint64_t start_bit, end_bit;
+    uint32_t n_sym;
+};
+class GzStreamInflater {
+   public:
+    GzStreamInflater(const uint8_t* data, size_t n, int device, uint64_t span_bytes = 0, uint64_t round_bytes = 0,
+                     std::vector<ChainEntry>* chain_log = nullptr);
+    ~GzStreamInflater();
+    GzStreamInflater(const GzStreamInflater&) = delete;
+    GzStreamInflater& operator=(const GzStreamInflater&) = delete;
+    long read(uint8_t* dst, size_t n);  // bytes produced (< n only at the end of the input), -1 on error
+    const char* error() const;
+    struct Impl;
+
+   private:
+    Impl* p_;
+};
+
 struct RawSource {  // decompressed byte stream of a plain or gzip (multi-member) file, read into caller memory
     int fd = -1;
     bool gz = false, file_eof = false, stream_end = false;

@@ -85,6 +85,10 @@ def lib():
         L.csq_gz_deflate_host.argtypes = [vp, C.c_uint64, vp, C.c_uint64, u64p]
         L.csq_gz_inflate_host.argtypes = [vp, C.c_uint64, vp, C.c_uint64, u64p, u64p]
         L.csq_pinflate_mem.argtypes = [vp, C.c_uint64, vp, C.c_uint64, C.c_int, C.c_uint64, u64p]
+        L.csq_gz_stream_inflate.argtypes = [i32, vp, C.c_uint64, vp, C.c_uint64, C.c_uint64, C.c_uint64, u64p]
+        L.csq_gz_stream_inflate_host.argtypes = [vp, C.c_uint64, vp, C.c_uint64, C.c_uint64, C.c_uint64, u64p]
+        L.csq_gz_stream_chain.argtypes = [u64p, C.c_uint64]
+        L.csq_gz_stream_chain.restype = C.c_uint64
     if hasattr(L, "csq_synth_batch"):
         L.csq_synth_batch.argtypes = [C.POINTER(A.csq_synth), C.c_uint64, u32, i32, C.POINTER(A.csq_batch_in)]
         L.csq_synth_free.restype = None
@@ -419,6 +423,34 @@ def pinflate(data: bytes, capacity: int, threads: int = 4, span_bytes: int = 0) 
     n = C.c_uint64(0)
     check(lib().csq_pinflate_mem(src.ctypes.data, len(data), out.ctypes.data, capacity, threads, span_bytes, C.byref(n)))
     return out[: n.value].tobytes()
+
+
+def _gz_stream(call, data: bytes, capacity: int, span_bytes: int, round_bytes: int, chain: bool):
+    src = np.frombuffer(bytes(data) + b"\0" * 16, dtype=np.uint8)
+    out = np.empty(max(capacity, 1), dtype=np.uint8)
+    n = C.c_uint64(0)
+    check(call(src.ctypes.data, len(data), out.ctypes.data, capacity, span_bytes, round_bytes, C.byref(n)))
+    text = out[: n.value].tobytes()
+    if not chain:
+        return text
+    k = lib().csq_gz_stream_chain(None, 0)
+    arr = np.zeros(3 * max(k, 1), dtype=np.uint64)
+    lib().csq_gz_stream_chain(arr.ctypes.data_as(C.POINTER(C.c_uint64)), k)
+    return text, [tuple(int(v) for v in arr[3 * i: 3 * i + 3]) for i in range(k)]
+
+
+def gz_stream_inflate(data: bytes, capacity: int, device: int = 0, span_bytes: int = 0, round_bytes: int = 0,
+                      chain: bool = False):
+    """An ordinary gzip file in memory through the device decoder (``csq_gz_stream_inflate``).  chain=True also returns
+    the decode chain: (start bit, end bit, symbols) of every span in file order."""
+    def call(*a):
+        return lib().csq_gz_stream_inflate(device, *a)
+    return _gz_stream(call, data, capacity, span_bytes, round_bytes, chain)
+
+
+def gz_stream_inflate_host(data: bytes, capacity: int, span_bytes: int = 0, round_bytes: int = 0, chain: bool = False):
+    """The device decoder's host twin (``csq_gz_stream_inflate_host``), as gz_stream_inflate."""
+    return _gz_stream(lib().csq_gz_stream_inflate_host, data, capacity, span_bytes, round_bytes, chain)
 
 
 def gz_inflate_host(data: bytes, capacity: int):

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define CSQ_ABI_VERSION 3
+#define CSQ_ABI_VERSION 4
 
 typedef enum csq_status {
     CSQ_OK = 0,
@@ -383,6 +383,19 @@ int csq_gz_inflate_host(const uint8_t* src, uint64_t n, uint8_t* dst, uint64_t c
  * without BGZF framing): a whole gzip file in memory -> text.  span_bytes: compressed bytes per thread and round
  * (0: default); tests use small values. */
 int csq_pinflate_mem(const uint8_t* src, uint64_t n, uint8_t* dst, uint64_t cap, int threads, uint64_t span_bytes, uint64_t* out_n);
+/* The device decoder of ordinary gzip files (csrc/gz_stream.cu; the device counterpart of csq_pinflate_mem, which the
+ * file driver keeps using - DESIGN.md section 4.6): a whole gzip file in memory -> text, decoded on `device`.  The stream is decoded in rounds of
+ * `round_bytes` compressed bytes, each cut into spans of `span_bytes` (0: the defaults, 64 MiB and 128 KiB); tests use
+ * small values.  CSQ_ERR_IO with a message for damaged, truncated or trailing-garbage input and CRC-32 / ISIZE
+ * mismatches, CSQ_ERR_CAPACITY when the text does not fit in `cap`. */
+int csq_gz_stream_inflate(int device, const uint8_t* src, uint64_t n, uint8_t* dst, uint64_t cap, uint64_t span_bytes,
+                          uint64_t round_bytes, uint64_t* out_n);
+/* The same decoder's host twin (the same search, decode, window and resolve code with one lane; CPU tests). */
+int csq_gz_stream_inflate_host(const uint8_t* src, uint64_t n, uint8_t* dst, uint64_t cap, uint64_t span_bytes,
+                               uint64_t round_bytes, uint64_t* out_n);
+/* The decode chain of the calling thread's last csq_gz_stream_inflate(_host) call: (start bit, end bit, symbols) of every
+ * span in file order, up to max_entries triples into out.  Returns the number of spans (tests). */
+uint64_t csq_gz_stream_chain(uint64_t* out, uint64_t max_entries);
 /* SoA batch -> FASTQ text of one mate ("@name\nseq\n+\nqual\n"), for tests and benchmarks. */
 int csq_format_fastq(const csq_mate_in* mate, uint32_t n_reads, uint8_t* out, uint64_t capacity,
                      uint64_t* bytes);
